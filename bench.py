@@ -9,12 +9,13 @@ metric = BASELINE.json configs[2] at one bit width) over tensors already residen
             host<->device copies inside the timing.
 `calib_wallclock` = the public `HessianQuantCalibrator(...).batching_quant_calib()` (capture + search + gather), the
             equivalent of what example/test_all.py:31-34 times.
-`reference_gpu` = the UNMODIFIED reference classes (baseline/_ref) on the same GPU, one layer per type, one round.
+`reference_gpu` = the UNMODIFIED reference classes (oracle/_ref) on the same GPU, one layer per type, one round.
 `cpu_baseline` / `--impl reference` = the reference classes on the host cores (bounded sample, see below).
 
   python bench.py --gpus 1 --steps 3 --warmup 3
   torchrun ... bench.py --gpus N ...          (layer-sharded, one all_gather of the step sizes per step)
   python bench.py --impl reference            (reference on the host cores)
+  python bench.py ... --dump-outputs DIR      (the step sizes of the last timed step as DIR/<module>.<name>.npy)
 """
 import argparse
 import ctypes
@@ -28,6 +29,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True                 # the tree may be read-only: nothing is written there
 os.environ.setdefault("TQDM_DISABLE", "1")
 if os.environ.get("NCCL_DEBUG", "VERSION").upper() == "VERSION":
     os.environ["NCCL_DEBUG"] = "NONE"          # keep stdout to the one JSON line (NCCL prints its version banner there)
@@ -53,6 +55,8 @@ def parse():
     ap.add_argument("--no-ref-gpu", action="store_true")
     ap.add_argument("--no-wallclock", action="store_true")
     ap.add_argument("--cpu-eq-n", type=int, default=20, help="candidates per search step of the CPU reference sample")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the step sizes the last timed step chose, one float32 "
+                    "DIR/<module>.<name>.npy per array, to compare two builds output for output")
     return ap.parse_args()
 
 
@@ -137,6 +141,19 @@ def build_workload(a, device, rank, world):
     return net, wrapped, work, owner, names, cal
 
 
+def dump_outputs(wrapped, out_dir):
+    """The arrays calibration_step2() leaves on every wrapped module (w_interval, a_interval, A_interval, B_interval,
+    split) as float32 .npy files."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, m in wrapped.items():
+        for key in ("w_interval", "a_interval", "A_interval", "B_interval", "split"):
+            v = getattr(m, key, None)
+            if v is not None:
+                arr = torch.as_tensor(v).detach().float().cpu().numpy()
+                np.save(os.path.join(out_dir, f"{name}.{key}.npy"), arr)
+
+
 def run_module(m, t):
     """One module's search through the reference-facing call, tensors already on the device."""
     if "x" in t:
@@ -204,7 +221,7 @@ def layer_types(a):
 
 
 def reference_rates(a, on_gpu, eq_n, only=None):
-    """Times the reference classes (oracle/ref_harness -> baseline/_ref; falls back to the oracle port) on one seeded
+    """Times the reference classes (oracle/ref_harness -> oracle/_ref; falls back to the oracle port) on one seeded
     synthetic layer of every type at the workload's sizes.  GPU: the whole calibration_step2() of one round, eq_n=100,
     the reference's own H2D copies included.  CPU: eq_n candidates per search step, the weight search of a Linear layer
     interrupted after one column block (+ one activation step).  Returns {type: (seconds, units)} and the kind."""
@@ -304,7 +321,7 @@ def reference_cpu_main(a):
             per_step.append({"value": round(v, 3), "job_s": round(job_s, 1), "sample_s": round(sum(s for s, _ in samples.values()), 2),
                              "rates": {k: round(r, 3) for k, r in rates.items()}})
     value = statistics.median(vals)
-    sample = (f"{'unmodified reference classes (baseline/_ref)' if kind == 'reference' else 'oracle port'} on {cores} threads "
+    sample = (f"{'unmodified reference classes (oracle/_ref)' if kind == 'reference' else 'oracle port'} on {cores} threads "
               f"(physical cores, torch.set_num_threads): one seeded synthetic layer per type (qkv, proj, fc1, fc2, head, matmul1, matmul2) at "
               f"the workload's sizes; Linear: one column block of the weight search + the activation search, {a.cpu_eq_n} candidates "
               f"each; MatMul: calibration_step2 with eq_n={a.cpu_eq_n}, one round; extrapolated by unit counts to the whole job; "
@@ -388,6 +405,8 @@ def main():
         dist.all_reduce(tmax, op=dist.ReduceOp.MAX)
     ms = float(tmax.item())
     value = total_units * a.steps / (ms / 1e3)
+    if a.dump_outputs and rank == 0:
+        dump_outputs(wrapped, a.dump_outputs)          # after the gather every rank holds every module's step sizes
 
     # ---- the public calibrator: capture + search + gather (what example/test_all.py:31-34 times)
     wallclock = None

@@ -1,16 +1,15 @@
 """Run the UNMODIFIED reference classes (TEST / BASELINE INFRASTRUCTURE ONLY).
 
 Imports the reference's `quant_layers`, `utils.quant_calib`, `utils.net_wrap`, `configs.PTQ4ViT` from
-baseline/_ref (staged by oracle/stage_ref.py; travels to the GPU box) or, in the dev container, straight from
-/root/reference.  `timm` is not installed offline: a stub module tree provides the two class names
+oracle/_ref (staged by oracle/stage_ref.py) or straight from the tree named by $PTQ4VIT_REFERENCE.  `timm` is not installed offline: a stub module tree provides the two class names
 `utils/models.py` imports.  On a machine without a GPU the reference's hard-coded `.cuda()` calls
 (quant_layers/linear.py:391, :461-464; quant_layers/matmul.py:428, :493-498) are made the identity by a
-harness-only shim; on the B200 box the reference runs unmodified on the GPU.
+harness-only shim; on a GPU the reference runs unmodified.
 
 Score tables are captured by spying on argmax: every search step of the reference calls it exactly once on its
 similarity table (linear.py:493, :531; matmul.py:520, :561, :626).
 
-Only tests/, bench.py's reference legs and tests/golden/make_*.py import this file.
+Only bench.py's reference legs, tests/golden/make_*.py and tests that need no reference tree import this file.
 """
 import contextlib
 import os
@@ -20,15 +19,15 @@ import types
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-STAGED = os.path.join(ROOT, "baseline", "_ref")
+STAGED = os.path.join(ROOT, "oracle", "_ref")
 _ref = None
 
 
 def reference_path():
     if os.path.isdir(os.path.join(STAGED, "quant_layers")):
         return STAGED
-    src = os.environ.get("PTQ4VIT_REFERENCE", "/root/reference")
-    if os.path.isdir(os.path.join(src, "quant_layers")):
+    src = os.environ.get("PTQ4VIT_REFERENCE", "")
+    if src and os.path.isdir(os.path.join(src, "quant_layers")):
         return src
     return None
 
@@ -79,7 +78,7 @@ def load():
         return _ref
     path = reference_path()
     if path is None:
-        raise RuntimeError("reference tree not found: stage it with `python oracle/stage_ref.py` (dev container)")
+        raise RuntimeError("reference tree not found: set $PTQ4VIT_REFERENCE or stage it with `python oracle/stage_ref.py`")
     if not torch.cuda.is_available():
         cpu_shim()
     _stub_timm()

@@ -1,11 +1,11 @@
 """The public calibrator end to end: `HessianQuantCalibrator(net, wrapped, loader, sequential, batch_size)
 .batching_quant_calib()` on a 2-block synthetic ViT, against
 
-  * the UNMODIFIED reference calibrator (utils/quant_calib.py:300-378 + utils/net_wrap.py + configs/PTQ4ViT.py from
-    baseline/_ref) running on the same GPU: captured x / y / grad tensors and every chosen step size;
-  * tests/golden/calib_tiny_vit.npz (the same reference run, CPU, dev container) -- the check that remains when the
-    staged tree is absent.  CPU and GPU capture numerics differ in the last bits, so near-tie picks may move by a grid
-    step: the comparison counts differing entries.
+  * the UNMODIFIED reference calibrator (utils/quant_calib.py:300-378 + utils/net_wrap.py + configs/PTQ4ViT.py) as
+    recorded running on a B200 (tests/golden/ref_calib_*.npz): captured x / y / grad tensors (a seeded sample of
+    their entries) and every chosen step size;
+  * tests/golden/calib_tiny_vit.npz (the same reference run on the CPU).  CPU and GPU capture numerics differ in the
+    last bits, so near-tie picks may move by a grid step: the comparison counts differing entries.
 
 Also: single-pass capture == the reference's one-sweep-per-module capture (SURVEY.md 8f rank 1), sequential=True works
 (gradients reach the modules behind an already quantized layer), QuantCalibrator.{parallel,sequential}_quant_calib and
@@ -21,6 +21,7 @@ import torch
 os.environ.setdefault("TQDM_DISABLE", "1")
 
 from oracle import ref_harness as RH
+from tests import _refgold as G
 
 pytestmark = pytest.mark.gpu
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "calib_tiny_vit.npz")
@@ -76,25 +77,23 @@ def _count_diff(got, ref, what, max_frac, max_steps=3):
 def _as_dict(npz, prefix):
     out = {}
     for k in npz.files:
-        p, name, key = k.split("|")
-        if p == prefix:
-            out.setdefault(name, {})[key] = torch.from_numpy(npz[k])
+        parts = k.split("|")
+        if len(parts) == 3 and parts[0] == prefix:
+            out.setdefault(parts[1], {})[parts[2]] = torch.from_numpy(npz[k])
     return out
 
 
 def test_batching_quant_calib_matches_reference_calibrator_on_gpu():
-    snap_ours, snap_ref = {}, {}
+    snap_ours = {}
     got, net, wrapped, cal = _ours(keep=snap_ours)
     assert cal.timings["single_pass"] and cal.timings["total_s"] > 0
-    if not RH.available():
-        pytest.skip("baseline/_ref not staged: covered by the golden comparison below")
-    ref, _, wrapped_r = RH.run_reference_calibrator(_net(), RH.tiny_images(), batch_size=4, sequential=False, snapshot=snap_ref)
-    # captured tensors: same net, same ops, same device
+    z = G.load("calib_vit")
+    ref = _as_dict(z, "iv")
+    # captured tensors: same net, same ops, same kind of device
     worst = 0.0
     for name, d in snap_ours.items():
         for key, t in d.items():
-            r = snap_ref[name][key].to(t.device)
-            err = float((t - r).abs().max() / (r.abs().max() + 1e-30))
+            err = G.sample_rel_err(z, "cap_", f"{name}|{key}", t.cpu())
             worst = max(worst, err)
             assert err < 1e-4, f"captured {name}.{key} differs from the reference's capture: {err:.2e}"
     bad, n = _count_diff(got, ref, "vs reference on GPU", max_frac=0.05)
@@ -108,17 +107,15 @@ def test_batching_quant_calib_matches_reference_calibrator_on_gpu():
 def test_swin_windowed_attention_and_reduction_match_reference_calibrator():
     """BASELINE.json configs[4] geometry in small: shifted windows, window attention MatMuls with the batch dimension
     images x windows (reference utils/models.py:28-56) and the `reduction` Linear of patch merging (utils/net_wrap.py:42)."""
-    if not RH.available():
-        pytest.skip("needs the staged reference (baseline/_ref)")
-    snap_ours, snap_ref = {}, {}
+    snap_ours = {}
     got, net, wrapped, cal = _ours(keep=snap_ours, kind="swin")
     assert any(n.endswith("downsample.reduction") for n in wrapped) and any("layers.0.blocks.1.attn.matmul1" == n for n in wrapped)
-    ref, _, _ = RH.run_reference_calibrator(_net("swin"), RH.tiny_images(), batch_size=4, sequential=False, snapshot=snap_ref)
+    z = G.load("calib_swin")
+    ref = _as_dict(z, "iv")
     assert set(ref) == set(got)
     for name, d in snap_ours.items():
         for key, t in d.items():
-            r = snap_ref[name][key].to(t.device)
-            assert float((t - r).abs().max()) <= 1e-5 * float(r.abs().max()) + 1e-30, f"captured {name}.{key}"
+            assert G.sample_rel_err(z, "cap_", f"{name}|{key}", t.cpu()) <= 1e-5, f"captured {name}.{key}"
     bad, n = _count_diff(got, ref, "swin vs reference on GPU", max_frac=0.05)
     print(f"[calibrator swin] {len(got)} modules (window attention + patch merging), {bad}/{n} step sizes differ")
 
@@ -144,11 +141,9 @@ def test_single_pass_capture_equals_per_module_capture():
 def test_sequential_calibration_runs_and_tracks_reference():
     got, net, wrapped, cal = _ours(sequential=True)
     assert not cal.timings["single_pass"]
-    ref = _as_dict(np.load(GOLD), "seq")
-    if RH.available():
-        ref, _, _ = RH.run_reference_calibrator(_net(), RH.tiny_images(), batch_size=4, sequential=True)
-    bad, n = _count_diff(got, ref, "sequential", max_frac=0.3)
-    print(f"[calibrator sequential] {bad}/{n} step sizes differ")
+    bad, n = _count_diff(got, _as_dict(G.load("calib_vit_sequential"), "iv"), "sequential", max_frac=0.3)
+    bad_cpu, _ = _count_diff(got, _as_dict(np.load(GOLD), "seq"), "sequential vs CPU golden", max_frac=0.3)
+    print(f"[calibrator sequential] {bad}/{n} step sizes differ from the GPU reference run, {bad_cpu} from the CPU one")
 
 
 def test_quant_calibrator_parallel_and_sequential_drivers():
@@ -209,46 +204,37 @@ def test_base_batching_quant_calib_l2():
     importlib.reload(cfg)
 
 
+def wrap_non_batching(net, lin, gelu, mm, sos, matmul_type):
+    """Replace every Linear / MatMul of `net` by the given non-batching classes (hessian metric, two rounds)."""
+    kw = dict(metric="hessian", eq_alpha=0.01, eq_beta=1.2, eq_n=100, search_round=2)
+    wrapped = {}
+    for name, m in list(net.named_modules()):
+        parent = net.get_submodule(name.rsplit(".", 1)[0]) if "." in name else net
+        leaf = name.rsplit(".", 1)[-1]
+        if isinstance(m, torch.nn.Linear):
+            q = (gelu if leaf == "fc2" else lin)(m.in_features, m.out_features, n_V=3 if leaf == "qkv" else 1, **kw)
+            q.weight.data = m.weight.data; q.bias = m.bias; q.to(m.weight.device)
+        elif isinstance(m, matmul_type):
+            q = (sos if leaf == "matmul2" else mm)(**kw)
+        else:
+            continue
+        setattr(parent, leaf, q); wrapped[name] = q
+    return wrapped
+
+
 def test_hessian_quant_calib_non_batching_driver_matches_reference():
     """HessianQuantCalibrator.quant_calib (reference :216-298): the non-batching driver -- per module one forward+backward
     sweep, then `calibration_step2(x)` / `(A, B)` of the NON-batching classes with the hessian metric -- against the
     reference's same driver on its own non-batching classes (Linear and MatMul modules; both nets wrapped by hand)."""
-    if not RH.available():
-        pytest.skip("needs the staged reference (baseline/_ref)")
-    import copy
     from ptq4vit_b200.quant_layers import linear as L, matmul as M
     from ptq4vit_b200.utils import quant_calib as Q
     from ptq4vit_b200.utils.models import MatMul
-    R = RH.load()
-    kw = dict(metric="hessian", eq_alpha=0.01, eq_beta=1.2, eq_n=100, search_round=2)
-
-    def wrap(net, lin, gelu, mm, sos, matmul_type):
-        wrapped = {}
-        for name, m in list(net.named_modules()):
-            parent = net.get_submodule(name.rsplit(".", 1)[0]) if "." in name else net
-            leaf = name.rsplit(".", 1)[-1]
-            if isinstance(m, torch.nn.Linear):
-                q = (gelu if leaf == "fc2" else lin)(m.in_features, m.out_features, n_V=3 if leaf == "qkv" else 1, **kw)
-                q.weight.data = m.weight.data; q.bias = m.bias; q.to(m.weight.device)
-            elif isinstance(m, matmul_type):
-                q = (sos if leaf == "matmul2" else mm)(**kw)
-            else:
-                continue
-            setattr(parent, leaf, q); wrapped[name] = q
-        return wrapped
-
     net = _net()
-    net_r = copy.deepcopy(net)
-    for mod in net_r.modules():
-        for leaf in ("matmul1", "matmul2"):
-            if hasattr(mod, leaf):
-                setattr(mod, leaf, R.models.MatMul())
-    ours = wrap(net, L.PTQSLQuantLinear, L.PostGeluPTQSLQuantLinear, M.PTQSLQuantMatMul, M.SoSPTQSLQuantMatMul, MatMul)
-    refs = wrap(net_r, R.linear.PTQSLQuantLinear, R.linear.PostGeluPTQSLQuantLinear, R.matmul.PTQSLQuantMatMul,
-                R.matmul.SoSPTQSLQuantMatMul, R.models.MatMul)
+    ours = wrap_non_batching(net, L.PTQSLQuantLinear, L.PostGeluPTQSLQuantLinear, M.PTQSLQuantMatMul, M.SoSPTQSLQuantMatMul, MatMul)
     Q.HessianQuantCalibrator(net, ours, RH.ListLoader(RH.tiny_images()), sequential=False, batch_size=4).quant_calib()
-    R.quant_calib.HessianQuantCalibrator(net_r, refs, RH.ListLoader(RH.tiny_images()), sequential=False, batch_size=4).quant_calib()
     torch.cuda.synchronize()
     assert all(m.calibrated and m.mode == "quant_forward" for m in ours.values())
-    bad, n = _count_diff(RH.collect_intervals(ours), RH.collect_intervals(refs), "non-batching hessian driver", max_frac=0.1)
+    ref = _as_dict(G.load("calib_non_batching"), "iv")
+    assert set(ref) == set(ours)
+    bad, n = _count_diff(RH.collect_intervals(ours), ref, "non-batching hessian driver", max_frac=0.1)
     print(f"[calibrator non-batching] {len(ours)} modules, {bad}/{n} step sizes differ")
