@@ -6,8 +6,8 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libptq4vit_b200.so")
-SOURCES = ["sweep_tc.cu", "sweep_simt.cu", "prep.cu", "gram.cu", "gram_gemm.cu", "linear_api.cu", "matmul_api.cu", "conv_api.cu",
-           "export.cu"]
+SOURCES = ["runtime.cu", "sweep_tc.cu", "sweep_simt.cu", "prep.cu", "gram.cu", "gram_gemm.cu", "linear_api.cu", "matmul_api.cu",
+           "conv_api.cu", "export.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden"]
 

@@ -119,3 +119,14 @@ extern "C" void p4v_set_error(const char* fmt, ...);
 // ---- kernel launchers shared between translation units ----------------------
 int p4v_launch_sweep_tc(const SweepParams& p, const P4VJob* host_jobs, int num_sms, cudaStream_t st);
 int p4v_launch_sweep_simt(const SweepParams& p, cudaStream_t st);
+
+// ---- library runtime (runtime.cu) -------------------------------------------
+void p4v_count_launch();     // every kernel launch of the library counts itself (p4v_launch_count)
+int p4v_num_sms();
+// one sweep launch on the kernel desc.kernel selects (P4V_KERNEL_*), counted and, while profiling is on, timed
+int p4v_run_sweep(const SweepParams& sp, const P4VJob* host_jobs, int kernel, cudaStream_t st);
+// live kernel timing: kinds of the record p4v_profile_collect_kinds reports
+enum { P4V_PROF_SWEEP_BF16 = 0, P4V_PROF_SWEEP_INT8 = 1, P4V_PROF_GRAM_GEMM = 2, P4V_PROF_KINDS = 3 };
+bool p4v_prof_on();
+void p4v_prof_begin(cudaStream_t st, cudaEvent_t* e0);
+void p4v_prof_end(cudaStream_t st, cudaEvent_t e0, int kind, double ops);

@@ -14,15 +14,10 @@
 #include <vector>
 
 #include "../../include/ptq4vit_b200.h"
+#include "plan.cuh"
 #include "prep.cuh"
 
-void p4v_count_launch();
-int p4v_run_sweep(const SweepParams& sp, const P4VJob* host_jobs, int kernel, cudaStream_t st);
-
 namespace {
-
-inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
-template <class T> T* at(void* ws, size_t off) { return reinterpret_cast<T*>(static_cast<uint8_t*>(ws) + off); }
 
 struct ConvPlan {
   p4v_conv_desc d;
@@ -47,31 +42,23 @@ int build_plan(const p4v_conv_desc* d, ConvPlan& p) {
   p.segW = {P4VSeg{0, p.K, 0, 0, 0.f, (float)-p.w_qmax, (float)(p.w_qmax - 1), 0, 0.f, 0, 0}};
   p.segC.clear();
   for (int t = 0; t < 3; ++t) p.segC.push_back(P4VSeg{0, p.K, t * p.kb * P4V_TILE, 0, 0.f, 0.f, 0.f, 0, 0.f, t + 1, 0});
-  p.factors.resize(d->eq_n + 1);
-  for (int i = 0; i <= d->eq_n; ++i) p.factors[i] = (float)(d->eq_alpha + i * (d->eq_beta - d->eq_alpha) / d->eq_n);
+  p.factors = candidate_factors(d->eq_alpha, d->eq_beta, d->eq_n);
   p.jobs.clear();
-  for (int t = 0; t < 3; ++t)
-    for (int b = 0; b < p.kb; b += P4V_JOB_KB) {
-      P4VJob j{};
-      const int len = std::min(P4V_JOB_KB, p.kb - b);
-      j.r_off = (uint32_t)b * P4V_TILE; j.c_off = (uint32_t)(t * p.kb + b) * P4V_TILE; j.kb = (uint8_t)len;
-      j.flags = P4V_JOB_RCAND | ((t == 0 && b == 0) ? P4V_JOB_FIRST : 0) | ((t == 2 && b + len >= p.kb) ? P4V_JOB_LAST : 0);
-      j.group = 0;
-      p.jobs.push_back(j);
-    }
-  size_t o = 0;
-  auto take = [&](size_t bytes) { size_t r = o; o = align_up(o + bytes, 256); return r; };
+  int n_jobs = 0;
+  for (int t = 0; t < 3; ++t)        // the three term products chain into one accumulator
+    push_jobs(p.jobs, 0, t * p.kb, p.kb, P4V_JOB_RCAND, 0, t == 0, t == 2, n_jobs);
+  Carver w;
   const int n_c = d->eq_n;
-  p.o_factors = take((n_c + 1) * 4); p.o_keys = take((p.O + 1) * 4);
-  p.o_d0 = take(p.O * 4); p.o_d = take(p.O * 4); p.o_gscale = take(4); p.o_ones = take(4);
-  p.o_scores = take((size_t)n_c * p.O * 8); p.o_best = take(p.O * 4);
-  p.o_candA = take((size_t)n_c * 4); p.o_candB = take(4); p.o_fix = take(4);
-  p.o_jobs = take(p.jobs.size() * sizeof(P4VJob)); p.o_segW = take(sizeof(P4VSeg)); p.o_segC = take(3 * sizeof(P4VSeg));
-  p.o_partial = take((size_t)p.P * p.tiles_o * p.tiles_l * n_c * 256 * 4);
-  p.o_Wcand = take((size_t)n_c * p.tiles_o * P4V_TILE * p.kb);
-  p.o_Cimg = take((size_t)p.P * p.tiles_l * P4V_TILE * 3 * p.kb);
-  p.o_Y = take((size_t)p.P * p.O * p.L * 4); p.o_G = take((size_t)p.P * p.O * p.L * 4);
-  p.total = o;
+  p.o_factors = w.take((n_c + 1) * 4); p.o_keys = w.take((p.O + 1) * 4);
+  p.o_d0 = w.take(p.O * 4); p.o_d = w.take(p.O * 4); p.o_gscale = w.take(4); p.o_ones = w.take(4);
+  p.o_scores = w.take((size_t)n_c * p.O * 8); p.o_best = w.take(p.O * 4);
+  p.o_candA = w.take((size_t)n_c * 4); p.o_candB = w.take(4); p.o_fix = w.take(4);
+  p.o_jobs = w.take(p.jobs.size() * sizeof(P4VJob)); p.o_segW = w.take(sizeof(P4VSeg)); p.o_segC = w.take(3 * sizeof(P4VSeg));
+  p.o_partial = w.take((size_t)p.P * p.tiles_o * p.tiles_l * n_c * 256 * 4);
+  p.o_Wcand = w.take((size_t)n_c * p.tiles_o * P4V_TILE * p.kb);
+  p.o_Cimg = w.take((size_t)p.P * p.tiles_l * P4V_TILE * 3 * p.kb);
+  p.o_Y = w.take((size_t)p.P * p.O * p.L * 4); p.o_G = w.take((size_t)p.P * p.O * p.L * 4);
+  p.total = w.total;
   return 0;
 }
 
@@ -112,11 +99,7 @@ __global__ void conv_fill_kernel(float* candA, const float* factors, int n, floa
 }  // namespace
 
 extern "C" int p4v_conv_workspace_bytes(const p4v_conv_desc* d, size_t* bytes) {
-  ConvPlan p; int rc = build_plan(d, p);
-  if (rc) return rc;
-  P4V_REQUIRE(bytes != nullptr, "null output");
-  *bytes = p.total;
-  return 0;
+  return plan_workspace_bytes(build_plan, d, bytes);
 }
 
 extern "C" int p4v_conv_calibrate(const p4v_conv_desc* d, const float* cols, const float* weight, const float* bias,
@@ -128,10 +111,8 @@ extern "C" int p4v_conv_calibrate(const p4v_conv_desc* d, const float* cols, con
   P4V_REQUIRE(!d->has_bias || bias, "conv_calibrate: has_bias set but bias is null");
   P4V_REQUIRE(workspace_bytes >= p.total, "conv_calibrate: workspace too small (%zu < %zu)", workspace_bytes, p.total);
   cudaStream_t st = (cudaStream_t)stream;
-  P4V_CUDA_OK(cudaMemcpyAsync(at<void>(ws, p.o_factors), p.factors.data(), p.factors.size() * 4, cudaMemcpyHostToDevice, st));
-  P4V_CUDA_OK(cudaMemcpyAsync(at<void>(ws, p.o_jobs), p.jobs.data(), p.jobs.size() * sizeof(P4VJob), cudaMemcpyHostToDevice, st));
-  P4V_CUDA_OK(cudaMemcpyAsync(at<void>(ws, p.o_segW), p.segW.data(), sizeof(P4VSeg), cudaMemcpyHostToDevice, st));
-  P4V_CUDA_OK(cudaMemcpyAsync(at<void>(ws, p.o_segC), p.segC.data(), 3 * sizeof(P4VSeg), cudaMemcpyHostToDevice, st));
+  if ((rc = upload(ws, p.o_factors, p.factors, st)) || (rc = upload(ws, p.o_jobs, p.jobs, st)) ||
+      (rc = upload(ws, p.o_segW, p.segW, st)) || (rc = upload(ws, p.o_segC, p.segC, st))) return rc;
   // min-max step size per output channel (conv.py:487) and the gradient scale
   int* keys = at<int>(ws, p.o_keys);
   if ((rc = p4v_keys_reset(keys, p.O + 1, st))) return rc;

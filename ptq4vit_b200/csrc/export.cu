@@ -10,8 +10,6 @@
 #include "prep.cuh"
 #include "../../include/ptq4vit_b200.h"
 
-void p4v_count_launch();
-
 namespace {
 
 struct ExportArgs {

@@ -16,8 +16,6 @@
 // evaluation and the small reductions.
 #include "gram.cuh"
 
-void p4v_count_launch();
-
 namespace {
 
 __device__ __forceinline__ float fq_dev(float w, float delta, float lo, float hi) {
@@ -334,7 +332,6 @@ int p4v_gram_update(const GramUpdateArgs& a, cudaStream_t st) {
   return launch_update<64>(a, st);
 }
 int p4v_gram_update_splits(int O, int M) {      // token splits: one wave of two blocks per SM
-  int p4v_num_sms();
   const int cb = p4v_cdiv(O, 256);
   int s = (2 * p4v_num_sms()) / cb;
   const int max_s = p4v_cdiv(M, GRAM_BM);

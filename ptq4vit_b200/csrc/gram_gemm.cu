@@ -17,12 +17,6 @@
 #include "gram.cuh"
 #include <cstdio>
 
-void p4v_count_launch();
-int p4v_num_sms();
-bool p4v_prof_on();
-void p4v_prof_begin(cudaStream_t st, cudaEvent_t* e0);
-void p4v_prof_end(cudaStream_t st, cudaEvent_t e0, int kind, double ops);
-
 namespace {
 
 constexpr int kThreads = 64 + 256;
@@ -234,7 +228,7 @@ int p4v_gram_gemm(const GramGemmArgs& a, cudaStream_t st) {
   if (p4v_prof_on()) p4v_prof_begin(st, &e0);
   gram_gemm_kernel<<<grid, kThreads, smem, st>>>(a); p4v_count_launch();
   // three bf16 term products per (output channel, pair, token): 128x256 tiles over term_bytes/2 tokens
-  if (p4v_prof_on()) p4v_prof_end(st, e0, 2, 3.0 * 2.0 * 128.0 * 256.0 * (double)tiles * (double)(a.term_bytes / 2));
+  if (p4v_prof_on()) p4v_prof_end(st, e0, P4V_PROF_GRAM_GEMM, 3.0 * 2.0 * 128.0 * 256.0 * (double)tiles * (double)(a.term_bytes / 2));
   P4V_CUDA_OK(cudaGetLastError());
   return 0;
 }

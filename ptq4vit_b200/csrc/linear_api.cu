@@ -1,117 +1,15 @@
 // C-ABI for the Linear scale-factor search: host-side planning (segments, jobs,
 // workspace carving) + the per-step launch sequence.  See include/ptq4vit_b200.h.
 #include <algorithm>
-#include <cstdarg>
-#include <cstdio>
-#include <cstring>
 #include <cstdlib>
 #include <vector>
 
 #include "../../include/ptq4vit_b200.h"
+#include "plan.cuh"
 #include "prep.cuh"
 #include "gram.cuh"
 
-int p4v_num_sms();
-
-// ---------------------------------------------------------------- error / misc
-static thread_local char g_err[512] = "";
-static long long g_launches = 0;
-extern "C" __attribute__((visibility("default"))) void p4v_set_error(const char* fmt, ...) {
-  va_list ap; va_start(ap, fmt); vsnprintf(g_err, sizeof(g_err), fmt, ap); va_end(ap);
-}
-extern "C" const char* p4v_last_error(void) { return g_err; }
-extern "C" int p4v_version(void) { return 100; }
-extern "C" long long p4v_launch_count(void) { return g_launches; }
-void p4v_count_launch() { ++g_launches; }
-
-// ---- live kernel timing (bench.py's roofline) ---------------------------------
-// While enabled every tensor-core launch (slab sweep, Gram GEMM) is bracketed by CUDA events on its own stream and
-// recorded with its kind and the tensor-core operations (2*MAC) it executes.
-enum { P4V_PROF_SWEEP_BF16 = 0, P4V_PROF_SWEEP_INT8 = 1, P4V_PROF_GRAM_GEMM = 2, P4V_PROF_KINDS = 3 };
-static bool g_prof = false;
-struct ProfRec { cudaEvent_t e0, e1; int kind; double ops; int n_cand, nfg, ncg, nfj, ncj, out; long long tiles; };
-static std::vector<ProfRec> g_prof_recs;
-static std::vector<cudaEvent_t> g_prof_pool;
-static cudaEvent_t prof_event() {
-  if (!g_prof_pool.empty()) { cudaEvent_t e = g_prof_pool.back(); g_prof_pool.pop_back(); return e; }
-  cudaEvent_t e; cudaEventCreate(&e); return e;
-}
-bool p4v_prof_on() { return g_prof; }
-void p4v_prof_begin(cudaStream_t st, cudaEvent_t* e0) { *e0 = prof_event(); cudaEventRecord(*e0, st); }
-void p4v_prof_end(cudaStream_t st, cudaEvent_t e0, int kind, double ops) {
-  cudaEvent_t e1 = prof_event(); cudaEventRecord(e1, st);
-  g_prof_recs.push_back(ProfRec{e0, e1, kind, ops, 0, 0, 0, 0, 0, 0, 0});
-}
-extern "C" int p4v_profile_enable(int on) { g_prof = on != 0; return 0; }
-// out[0..2] ms per kind (bf16 sweep, int8 sweep, Gram GEMM), out[3..5] executed ops, out[6..8] launches,
-// out[9..11] the longest single launch: ms, ops, kind.  Synchronises the recorded events and clears the record.
-extern "C" int p4v_profile_collect_kinds(double* out, int n) {
-  P4V_REQUIRE(out && n >= 12, "profile_collect_kinds: need 12 doubles");
-  for (int i = 0; i < 12; ++i) out[i] = 0.0;
-  static const bool log_each = getenv("P4V_PROFILE_LOG") != nullptr;   // debug: one stderr line per launch
-  for (auto& r : g_prof_recs) {
-    P4V_CUDA_OK(cudaEventSynchronize(r.e1));
-    float t = 0.f;
-    P4V_CUDA_OK(cudaEventElapsedTime(&t, r.e0, r.e1));
-    out[r.kind] += t; out[3 + r.kind] += r.ops; out[6 + r.kind] += 1.0;
-    if (t > out[9]) { out[9] = t; out[10] = r.ops; out[11] = r.kind; }
-    if (log_each)
-      fprintf(stderr, "[p4v launch] %8.1f us kind=%d cand=%d fixed_groups=%d cand_groups=%d fixed_jobs=%d cand_jobs=%d out=%d tiles=%lld  %.1f TOP/s\n",
-              t * 1e3, r.kind, r.n_cand, r.nfg, r.ncg, r.nfj, r.ncj, r.out, r.tiles, r.ops / (t * 1e-3) / 1e12);
-    g_prof_pool.push_back(r.e0); g_prof_pool.push_back(r.e1);
-  }
-  g_prof_recs.clear();
-  return 0;
-}
-extern "C" int p4v_profile_collect(double* sweep_ms, long long* sweep_launches, double* executed_ops) {
-  double o[12];
-  int rc = p4v_profile_collect_kinds(o, 12);
-  if (rc) return rc;
-  if (sweep_ms) *sweep_ms = o[0] + o[1];
-  if (sweep_launches) *sweep_launches = (long long)(o[6] + o[7]);
-  if (executed_ops) *executed_ops = o[3] + o[4];
-  return 0;
-}
-// tensor-core work of one sweep launch: every job multiplies a 128x128 tile over kb bytes of K
-static double sweep_ops(const SweepParams& sp, const P4VJob* host_jobs) {
-  double kf = 0.0, kc = 0.0;
-  const double ew = sp.is_int8 ? 1.0 : 2.0;
-  for (int j = 0; j < sp.n_fixed_jobs; ++j) kf += host_jobs[j].kb * p4v_job_nsub(host_jobs[j]) / ew;
-  for (int j = 0; j < sp.n_cand_jobs; ++j) kc += host_jobs[sp.n_fixed_jobs + j].kb * p4v_job_nsub(host_jobs[sp.n_fixed_jobs + j]) / ew;
-  const double tiles = (double)sp.P * sp.tiles_m * sp.tiles_n;
-  return 2.0 * P4V_TILE * P4V_TILE * tiles * (kf + kc * sp.n_cand);
-}
-static long long* g_trace = nullptr;
-extern "C" __attribute__((visibility("default"))) int p4v_debug_trace(void* dev_ptr) { g_trace = (long long*)dev_ptr; return 0; }
-int p4v_run_sweep(const SweepParams& sp_in, const P4VJob* host_jobs, int kernel, cudaStream_t st) {
-  SweepParams sp = sp_in; sp.trace = g_trace;
-  ++g_launches;
-  cudaEvent_t e0 = nullptr;
-  if (g_prof) p4v_prof_begin(st, &e0);
-  int rc = kernel == P4V_KERNEL_SIMT ? p4v_launch_sweep_simt(sp, st) : p4v_launch_sweep_tc(sp, host_jobs, p4v_num_sms(), st);
-  if (g_prof) {
-    p4v_prof_end(st, e0, sp.is_int8 ? P4V_PROF_SWEEP_INT8 : P4V_PROF_SWEEP_BF16, sweep_ops(sp, host_jobs));
-    ProfRec& r = g_prof_recs.back();
-    r.n_cand = sp.n_cand; r.nfg = sp.n_fixed_groups; r.ncg = sp.n_cand_groups; r.nfj = sp.n_fixed_jobs; r.ncj = sp.n_cand_jobs;
-    r.out = sp.out != nullptr; r.tiles = (long long)sp.P * sp.tiles_m * sp.tiles_n;
-  }
-  return rc;
-}
-
-int p4v_num_sms();
-int p4v_num_sms() {
-  static int sms = 0;
-  if (sms == 0) {
-    int dev = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess) return 148;
-    if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || sms <= 0) sms = 148;
-  }
-  return sms;
-}
-
 namespace {
-
-inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
 struct BSeg { int k0, klen, h, a, kb; int woff, xoff_p, xoff_n, xcoff; };   // offsets: bytes in the padded row
 struct Step { int job_off, nfj, ncj, nfg, ncg, meta_fix, meta_cand, commit_off, ncommit, commit_chunks; };
@@ -124,7 +22,7 @@ struct LinPlan {
   std::vector<BSeg> segs;
   int KB_W, KB_X, KB_Xc;
   std::vector<P4VJob> jobs; std::vector<GroupMeta> metas; std::vector<CommitSeg> commits;
-  std::vector<P4VSeg> segsW, segsX, segsXc;
+  std::vector<P4VSeg> segsW, segsX, segsXc, segsG;
   std::vector<Step> wsteps, xsteps;
   Step fwd;   // quant_forward: every segment is a fixed group
   // normal-equation W search (gram.cu)
@@ -137,33 +35,6 @@ struct LinPlan {
   size_t o_factors, o_keys, o_dW0, o_dW, o_dX0, o_dX, o_gscale, o_scores, o_best, o_fix, o_candA, o_candB, o_jobs,
       o_metas, o_segsW, o_segsX, o_segsXc, o_commits, o_partial, o_Wcur, o_Xcur, o_Wcand, o_Xcand, total;
 };
-
-void add_group(LinPlan& p, int r_off_bytes, int c_off_bytes, int kb, uint8_t src_flags, int group_idx, int& njobs) {
-  for (int b = 0; b < kb; b += P4V_JOB_KB) {
-    P4VJob j{};
-    const int len = std::min(P4V_JOB_KB, kb - b);
-    j.r_off = (uint32_t)(r_off_bytes + b) * P4V_TILE;
-    j.c_off = (uint32_t)(c_off_bytes + b) * P4V_TILE;
-    j.kb = (uint8_t)len;
-    j.flags = src_flags | (b == 0 ? P4V_JOB_FIRST : 0) | (b + len >= kb ? P4V_JOB_LAST : 0);
-    j.group = (uint8_t)group_idx;
-    p.jobs.push_back(j);
-    ++njobs;
-  }
-}
-
-// Candidate jobs whose row operand does not depend on the candidate (W steps): keep it resident in shared memory.
-void mark_resident(LinPlan& p, const Step& st) {
-  uint32_t total = 0;
-  for (int j = 0; j < st.ncj; ++j) total += (uint32_t)p.jobs[st.job_off + st.nfj + j].kb * P4V_TILE;
-  if (total == 0 || total > 60 * 1024) return;
-  uint32_t off = 0;
-  for (int j = 0; j < st.ncj; ++j) {
-    P4VJob& jb = p.jobs[st.job_off + st.nfj + j];
-    if (jb.flags & P4V_JOB_RCAND) return;
-    jb.flags |= P4V_JOB_RRES; jb.res_off = off; off += (uint32_t)jb.kb * P4V_TILE;
-  }
-}
 
 // Merge runs of single-job accumulator groups whose K slabs are adjacent in BOTH operand images into one
 // stage load with several sub-accumulators (one bulk copy / one stage handshake for up to 128 bytes of K).
@@ -217,9 +88,7 @@ int build_plan(const p4v_linear_desc* d, LinPlan& p, bool with_search) {
   cuts.erase(std::unique(cuts.begin(), cuts.end()), cuts.end());
   int min_len = p.K;
   for (size_t i = 0; i + 1 < cuts.size(); ++i) min_len = std::min(min_len, cuts[i + 1] - cuts[i]);
-  if (d->operand == P4V_OPERAND_INT8) p.i8 = true;
-  else if (d->operand == P4V_OPERAND_BF16) p.i8 = false;
-  else p.i8 = min_len >= 64;     // short slabs are epilogue bound: integer-valued bf16 saves the int->float converts (measured)
+  p.i8 = use_int8(d->operand, min_len);
   p.ew = p.i8 ? 1 : 2;
   p.segs.clear();
   int off = 0;
@@ -238,7 +107,7 @@ int build_plan(const p4v_linear_desc* d, LinPlan& p, bool with_search) {
   P4V_REQUIRE((size_t)p.KB_X * P4V_TILE < (1ull << 32), "linear: in_features too large");
 
   // quantisation segment tables
-  p.segsW.clear(); p.segsX.clear(); p.segsXc.clear();
+  p.segsW.clear(); p.segsX.clear(); p.segsXc.clear(); p.segsG.clear();
   for (auto& s : p.segs) {
     P4VSeg w{s.k0, s.klen, s.woff * P4V_TILE, s.h, 0.f, (float)-p.w_qmax, (float)(p.w_qmax - 1), 0, 0.f, 0, 0};
     p.segsW.push_back(w);
@@ -253,16 +122,14 @@ int build_plan(const p4v_linear_desc* d, LinPlan& p, bool with_search) {
       p.segsX.push_back(n);
     }
 
-  // candidate factors (python floats -> fp32, linear.py:544-545)
-  p.factors.resize(d->eq_n + 1);
-  for (int i = 0; i <= d->eq_n; ++i) p.factors[i] = (float)(d->eq_alpha + i * (d->eq_beta - d->eq_alpha) / d->eq_n);
+  p.factors = candidate_factors(d->eq_alpha, d->eq_beta, d->eq_n);
 
   // steps
   p.jobs.clear(); p.metas.clear(); p.commits.clear(); p.wsteps.clear(); p.xsteps.clear();
   p.max_groups = 1;
   auto begin_step = [&](Step& st) { st = Step{}; st.job_off = (int)p.jobs.size(); st.commit_off = (int)p.commits.size(); };
   auto fixed_group = [&](Step& st, const BSeg& s, bool neg) {
-    add_group(p, neg ? s.xoff_n : s.xoff_p, s.woff, s.kb, 0, st.nfg, st.nfj);
+    push_jobs(p.jobs, neg ? s.xoff_n : s.xoff_p, s.woff, s.kb, 0, st.nfg, true, true, st.nfj);
     p.metas.push_back(GroupMeta{(short)s.h, (short)s.a, (short)(neg ? 1 : 0), 0});
     ++st.nfg;
   };
@@ -273,16 +140,16 @@ int build_plan(const p4v_linear_desc* d, LinPlan& p, bool with_search) {
       for (auto& s : p.segs) if (s.h != h) { fixed_group(st, s, false); if (p.twin) fixed_group(st, s, true); }
       st.meta_cand = (int)p.metas.size();
       for (auto& s : p.segs) if (s.h == h) {
-        add_group(p, s.xoff_p, s.woff, s.kb, P4V_JOB_CCAND, st.ncg, st.ncj);
+        push_jobs(p.jobs, s.xoff_p, s.woff, s.kb, P4V_JOB_CCAND, st.ncg, true, true, st.ncj);
         p.metas.push_back(GroupMeta{(short)s.h, (short)s.a, 0, 0}); ++st.ncg;
         if (p.twin) {
-          add_group(p, s.xoff_n, s.woff, s.kb, P4V_JOB_CCAND, st.ncg, st.ncj);
+          push_jobs(p.jobs, s.xoff_n, s.woff, s.kb, P4V_JOB_CCAND, st.ncg, true, true, st.ncj);
           p.metas.push_back(GroupMeta{(short)s.h, (short)s.a, 1, 0}); ++st.ncg;
         }
         p.commits.push_back(CommitSeg{s.woff * P4V_TILE, s.woff * P4V_TILE, s.kb});
         st.commit_chunks += s.kb / 16; ++st.ncommit;
       }
-      mark_resident(p, st);
+      mark_resident(p.jobs, st.job_off + st.nfj, st.ncj);
       batch_jobs(p, st.job_off, st.nfj);
       p.wsteps.push_back(st);
     }
@@ -292,7 +159,7 @@ int build_plan(const p4v_linear_desc* d, LinPlan& p, bool with_search) {
       for (auto& s : p.segs) { if (s.a != a) fixed_group(st, s, false); if (p.twin) fixed_group(st, s, true); }
       st.meta_cand = (int)p.metas.size();
       for (auto& s : p.segs) if (s.a == a) {
-        add_group(p, s.xcoff, s.woff, s.kb, P4V_JOB_RCAND, st.ncg, st.ncj);
+        push_jobs(p.jobs, s.xcoff, s.woff, s.kb, P4V_JOB_RCAND, st.ncg, true, true, st.ncj);
         p.metas.push_back(GroupMeta{(short)s.h, (short)s.a, 0, 0}); ++st.ncg;
         p.commits.push_back(CommitSeg{s.xcoff * P4V_TILE, s.xoff_p * P4V_TILE, s.kb});
         st.commit_chunks += s.kb / 16; ++st.ncommit;
@@ -300,7 +167,7 @@ int build_plan(const p4v_linear_desc* d, LinPlan& p, bool with_search) {
       {   // candidates change the row operand only: keep the tile's weight image resident when it fits
         int ncj = st.ncj; batch_jobs(p, st.job_off + st.nfj, ncj); st.ncj = ncj;
         batch_jobs(p, st.job_off, st.nfj);
-        if ((size_t)p.KB_W * P4V_TILE <= 100 * 1024 && getenv("P4V_NO_CRES") == nullptr)
+        if ((size_t)p.KB_W * P4V_TILE <= 100 * 1024)
           for (int j = 0; j < st.nfj + st.ncj; ++j) p.jobs[st.job_off + j].flags |= P4V_JOB_CRES;
       }
       p.xsteps.push_back(st);
@@ -323,30 +190,29 @@ int build_plan(const p4v_linear_desc* d, LinPlan& p, bool with_search) {
   p.max_groups = std::max(p.max_groups, p.fwd.nfg);
 
   // workspace carving
-  size_t o = 0;
-  auto take = [&](size_t bytes) { size_t r = o; o = align_up(o + bytes, 256); return r; };
+  Carver w;
   const int n_c = d->eq_n;
-  p.o_factors = take((n_c + 1) * 4);
-  p.o_keys = take((d->n_V * d->n_H + d->n_a + 1) * 4);
-  p.o_dW0 = take(d->n_V * d->n_H * 4); p.o_dW = take(d->n_V * d->n_H * 4);
-  p.o_dX0 = take(d->n_a * 4); p.o_dX = take(d->n_a * 4);
-  p.o_gscale = take(4);
-  p.o_scores = take((size_t)n_c * (p.nsg + d->n_V * (size_t)(1 + p4v_cdiv(p.crb_rows, 2))) * 8);
-  p.o_best = take(std::max(d->n_V, 1) * 4);
-  p.o_fix = take((size_t)p.max_groups * p.nsg * 4);
-  p.o_candA = take((size_t)n_c * p.nsg * 4);
-  p.o_candB = take((size_t)p.max_groups * p.nsg * 4);
-  p.o_jobs = take(p.jobs.size() * sizeof(P4VJob));
-  p.o_metas = take(p.metas.size() * sizeof(GroupMeta));
-  p.o_segsW = take(p.segsW.size() * sizeof(P4VSeg));
-  p.o_segsX = take(p.segsX.size() * sizeof(P4VSeg));
-  p.o_segsXc = take(p.segsXc.size() * sizeof(P4VSeg));
-  p.o_commits = take(std::max<size_t>(1, p.commits.size()) * sizeof(CommitSeg));
-  p.o_partial = take(with_search ? (size_t)p.tiles_m * p.tiles_o * n_c * 32 * 4 : 4);
-  p.o_Wcur = take((size_t)p.tiles_o * P4V_TILE * p.KB_W);
-  p.o_Xcur = take((size_t)p.tiles_m * P4V_TILE * p.KB_X);
-  p.o_Wcand = take(with_search ? (size_t)n_c * p.tiles_o * P4V_TILE * p.KB_W : 4);
-  p.o_Xcand = take(with_search ? (size_t)n_c * p.tiles_m * P4V_TILE * p.KB_Xc : 4);
+  p.o_factors = w.take((n_c + 1) * 4);
+  p.o_keys = w.take((d->n_V * d->n_H + d->n_a + 1) * 4);
+  p.o_dW0 = w.take(d->n_V * d->n_H * 4); p.o_dW = w.take(d->n_V * d->n_H * 4);
+  p.o_dX0 = w.take(d->n_a * 4); p.o_dX = w.take(d->n_a * 4);
+  p.o_gscale = w.take(4);
+  p.o_scores = w.take((size_t)n_c * (p.nsg + d->n_V * (size_t)(1 + p4v_cdiv(p.crb_rows, 2))) * 8);
+  p.o_best = w.take(std::max(d->n_V, 1) * 4);
+  p.o_fix = w.take((size_t)p.max_groups * p.nsg * 4);
+  p.o_candA = w.take((size_t)n_c * p.nsg * 4);
+  p.o_candB = w.take((size_t)p.max_groups * p.nsg * 4);
+  p.o_jobs = w.take(p.jobs.size() * sizeof(P4VJob));
+  p.o_metas = w.take(p.metas.size() * sizeof(GroupMeta));
+  p.o_segsW = w.take(p.segsW.size() * sizeof(P4VSeg));
+  p.o_segsX = w.take(p.segsX.size() * sizeof(P4VSeg));
+  p.o_segsXc = w.take(p.segsXc.size() * sizeof(P4VSeg));
+  p.o_commits = w.take(std::max<size_t>(1, p.commits.size()) * sizeof(CommitSeg));
+  p.o_partial = w.take(with_search ? (size_t)p.tiles_m * p.tiles_o * n_c * 32 * 4 : 4);
+  p.o_Wcur = w.take((size_t)p.tiles_o * P4V_TILE * p.KB_W);
+  p.o_Xcur = w.take((size_t)p.tiles_m * P4V_TILE * p.KB_X);
+  p.o_Wcand = w.take(with_search ? (size_t)n_c * p.tiles_o * P4V_TILE * p.KB_W : 4);
+  p.o_Xcand = w.take(with_search ? (size_t)n_c * p.tiles_m * P4V_TILE * p.KB_Xc : 4);
   // normal-equation W search: narrow column blocks inside one activation chunk, plain (non twin) activations
   p.gram = false;
   {
@@ -361,39 +227,32 @@ int build_plan(const p4v_linear_desc* d, LinPlan& p, bool with_search) {
       p.g_tiles_p = p4v_cdiv(p.g_npairs * d->n_H, GRAM_PT); p.g_ldH = p.g_tiles_p * GRAM_PT;   // all column blocks side by side
       p.g_nmblk = p4v_gram_update_splits(p.O, p.M);
       const size_t KBg = 2 * (size_t)term;
-      p.o_E = take((size_t)p.M * p.O * 4);
-      p.o_XqT = take((size_t)p.K * p.g_Mp);
-      p.o_G2T = take((size_t)p.tiles_o * P4V_TILE * KBg);
-      p.o_Z = take((size_t)p.g_tiles_p * GRAM_PT * KBg);
-      p.o_H = take((size_t)p.O * p.g_ldH * 4);
-      p.o_Upart = take((size_t)p.g_nmblk * p.O * p.g_ks * 4);
-      p.o_E2part = take((size_t)p.g_nmblk * p.O * 4);
-      p.o_U = take((size_t)p.O * p.g_ks * 4); p.o_E2 = take((size_t)p.O * 4);
+      p.o_E = w.take((size_t)p.M * p.O * 4);
+      p.o_XqT = w.take((size_t)p.K * p.g_Mp);
+      p.o_G2T = w.take((size_t)p.tiles_o * P4V_TILE * KBg);
+      p.o_Z = w.take((size_t)p.g_tiles_p * GRAM_PT * KBg);
+      p.o_H = w.take((size_t)p.O * p.g_ldH * 4);
+      p.o_Upart = w.take((size_t)p.g_nmblk * p.O * p.g_ks * 4);
+      p.o_E2part = w.take((size_t)p.g_nmblk * p.O * 4);
+      p.o_U = w.take((size_t)p.O * p.g_ks * 4); p.o_E2 = w.take((size_t)p.O * 4);
       p.g_osplit = std::max(1, p4v_cdiv(p.crb_rows, 2)); p.g_opb = p4v_cdiv(p.crb_rows, p.g_osplit);
-      p.o_dprev = take((size_t)d->n_V * 4);
-      p.o_D = take((size_t)p.O * 64 * 4);
-      p.o_segsG = take(2 * sizeof(P4VSeg));
+      p.o_dprev = w.take((size_t)d->n_V * 4);
+      p.o_D = w.take((size_t)p.O * 64 * 4);
+      // (gs*g)^2 as two exact bf16 terms side by side in each row
+      p.segsG = {{0, p.M, 0, 0, 0.f, 0.f, 0.f, 0, 0.f, 1, 1}, {0, p.M, (int)(term * P4V_TILE), 0, 0.f, 0.f, 0.f, 0, 0.f, 2, 1}};
+      p.o_segsG = w.take(p.segsG.size() * sizeof(P4VSeg));
     }
   }
-  p.total = o;
+  p.total = w.total;
   return 0;
 }
 
-template <class T> T* at(void* ws, size_t off) { return reinterpret_cast<T*>(static_cast<uint8_t*>(ws) + off); }
-
 int upload_tables(const LinPlan& p, void* ws, cudaStream_t st) {
-  P4V_CUDA_OK(cudaMemcpyAsync(at<void>(ws, p.o_factors), p.factors.data(), p.factors.size() * 4, cudaMemcpyHostToDevice, st));
-  P4V_CUDA_OK(cudaMemcpyAsync(at<void>(ws, p.o_jobs), p.jobs.data(), p.jobs.size() * sizeof(P4VJob), cudaMemcpyHostToDevice, st));
-  P4V_CUDA_OK(cudaMemcpyAsync(at<void>(ws, p.o_metas), p.metas.data(), p.metas.size() * sizeof(GroupMeta), cudaMemcpyHostToDevice, st));
-  P4V_CUDA_OK(cudaMemcpyAsync(at<void>(ws, p.o_segsW), p.segsW.data(), p.segsW.size() * sizeof(P4VSeg), cudaMemcpyHostToDevice, st));
-  P4V_CUDA_OK(cudaMemcpyAsync(at<void>(ws, p.o_segsX), p.segsX.data(), p.segsX.size() * sizeof(P4VSeg), cudaMemcpyHostToDevice, st));
-  P4V_CUDA_OK(cudaMemcpyAsync(at<void>(ws, p.o_segsXc), p.segsXc.data(), p.segsXc.size() * sizeof(P4VSeg), cudaMemcpyHostToDevice, st));
-  if (!p.commits.empty())
-    P4V_CUDA_OK(cudaMemcpyAsync(at<void>(ws, p.o_commits), p.commits.data(), p.commits.size() * sizeof(CommitSeg), cudaMemcpyHostToDevice, st));
-  if (p.gram) {
-    P4VSeg sg[2] = {{0, p.M, 0, 0, 0.f, 0.f, 0.f, 0, 0.f, 1, 1}, {0, p.M, (int)(p.g_term_bytes * P4V_TILE), 0, 0.f, 0.f, 0.f, 0, 0.f, 2, 1}};
-    P4V_CUDA_OK(cudaMemcpyAsync(at<void>(ws, p.o_segsG), sg, sizeof(sg), cudaMemcpyHostToDevice, st));
-  }
+  int rc;
+  if ((rc = upload(ws, p.o_factors, p.factors, st)) || (rc = upload(ws, p.o_jobs, p.jobs, st)) ||
+      (rc = upload(ws, p.o_metas, p.metas, st)) || (rc = upload(ws, p.o_segsW, p.segsW, st)) ||
+      (rc = upload(ws, p.o_segsX, p.segsX, st)) || (rc = upload(ws, p.o_segsXc, p.segsXc, st)) ||
+      (rc = upload(ws, p.o_commits, p.commits, st)) || (rc = upload(ws, p.o_segsG, p.segsG, st))) return rc;
   return 0;
 }
 
@@ -464,37 +323,30 @@ int tables_for(const LinPlan& p, void* ws, const Step& s, int kind, int target, 
   return p4v_step_tables(tables_args(p, ws, s, kind, target), st);
 }
 
+// One search step: a W step (column block idx) or an X step (activation chunk idx).
 struct StepRef { bool is_w; int idx; };
 
-// One search step: [scale tables] -> sweep -> reduce -> select (+ tables of the next step) -> commit.
-int search_step(const LinPlan& p, void* ws, StepRef cur, const StepRef* next, bool tables_ready, const float* bias,
-                const float* y, const float* g, float* score_log, cudaStream_t st) {
-  const bool is_w = cur.is_w; const int idx = cur.idx;
-  const Step& s = is_w ? p.wsteps[idx] : p.xsteps[idx];
-  int rc;
-  if (!tables_ready && (rc = tables_for(p, ws, s, is_w ? 0 : 1, idx, st))) return rc;
-  SweepParams sp; fill_sweep(p, ws, s, sp);
-  sp.Y = y; sp.Gr = g; sp.bias = p.d.has_bias ? bias : nullptr;
-  sp.order = is_w ? 0 : 1;
-  if ((rc = run_sweep(p, s, sp, st))) return rc;
-  const int n_groups = is_w ? p.d.n_V : 1;
-  ReduceArgs r{};
-  r.partial = sp.partial; r.n_cand = p.d.eq_n; r.P = 1; r.tiles_m = p.tiles_m; r.tiles_n = p.tiles_o; r.order = sp.order;
-  r.mode = P4V_SG_COLUMN; r.n_keys = p.nsg; r.sums = at<double>(ws, p.o_scores);
-  if ((rc = p4v_reduce_scores(r, st))) return rc;
+const Step& step_of(const LinPlan& p, StepRef r) { return r.is_w ? p.wsteps[r.idx] : p.xsteps[r.idx]; }
+
+// Best candidate per row block (W step) / for the chunk (X step) from the score sums: the new step sizes.  The caller
+// sets how the score keys map to the groups (n_keys, keys_per_group) and what else the select does (d_prev, has_next).
+SelectArgs select_args(const LinPlan& p, void* ws, StepRef cur, float* score_log) {
   SelectArgs f{};
-  f.sums = r.sums; f.n_cand = p.d.eq_n; f.n_keys = p.nsg; f.n_groups = n_groups;
-  f.keys_per_group = (is_w && p.d.n_V > 1) ? p.crb_rows / P4V_CG : p.nsg;
-  f.inv_count = 1.0 / ((double)p.d.tokens * (double)(is_w ? p.crb_rows : p.O));
+  f.sums = at<double>(ws, p.o_scores); f.n_cand = p.d.eq_n; f.n_groups = cur.is_w ? p.d.n_V : 1;
+  f.inv_count = 1.0 / ((double)p.d.tokens * (double)(cur.is_w ? p.crb_rows : p.O));
   f.gscale = at<float>(ws, p.o_gscale); f.factors = at<float>(ws, p.o_factors);
-  if (is_w) { f.d0 = at<float>(ws, p.o_dW0); f.d = at<float>(ws, p.o_dW); f.d_stride = p.d.n_H; f.d_col = idx; }
-  else      { f.d0 = at<float>(ws, p.o_dX0); f.d = at<float>(ws, p.o_dX); f.d_stride = 0; f.d_col = idx; }
+  if (cur.is_w) { f.d0 = at<float>(ws, p.o_dW0); f.d = at<float>(ws, p.o_dW); f.d_stride = p.d.n_H; f.d_col = cur.idx; }
+  else          { f.d0 = at<float>(ws, p.o_dX0); f.d = at<float>(ws, p.o_dX); f.d_stride = 0; f.d_col = cur.idx; }
   f.best = at<int>(ws, p.o_best); f.score_log = score_log;
-  f.has_next = next != nullptr;
-  if (next) f.next = tables_args(p, ws, next->is_w ? p.wsteps[next->idx] : p.xsteps[next->idx], next->is_w ? 0 : 1, next->idx);
-  if ((rc = p4v_select_step(f, st))) return rc;
+  return f;
+}
+
+// Copy the chosen candidate's slabs of the step into the current operand image.
+CommitArgs commit_args(const LinPlan& p, void* ws, StepRef cur) {
+  const bool is_w = cur.is_w;
+  const Step& s = step_of(p, cur);
   CommitArgs c{};
-  c.best = f.best; c.n_groups = n_groups;
+  c.best = at<int>(ws, p.o_best); c.n_groups = is_w ? p.d.n_V : 1;
   c.cand = at<uint8_t>(ws, is_w ? p.o_Wcand : p.o_Xcand);
   c.cand_tile_bytes = (unsigned long long)P4V_TILE * (is_w ? p.KB_W : p.KB_Xc);
   c.cand_plane_stride = c.cand_tile_bytes * (is_w ? p.tiles_o : p.tiles_m);
@@ -503,7 +355,47 @@ int search_step(const LinPlan& p, void* ws, StepRef cur, const StepRef* next, bo
   c.P = 1; c.tiles = is_w ? p.tiles_o : p.tiles_m;
   c.rows_per_group = is_w ? p.crb_rows : 0; c.problem_groups = 0;
   c.segs = at<CommitSeg>(ws, p.o_commits) + s.commit_off; c.nseg = s.ncommit; c.commit_chunks = s.commit_chunks;
-  return p4v_commit_step(c, st);
+  return c;
+}
+
+// One search step: [scale tables] -> sweep -> reduce -> select (+ tables of the next step) -> commit.
+int search_step(const LinPlan& p, void* ws, StepRef cur, const StepRef* next, bool tables_ready, const float* bias,
+                const float* y, const float* g, float* score_log, cudaStream_t st) {
+  const bool is_w = cur.is_w;
+  const Step& s = step_of(p, cur);
+  int rc;
+  if (!tables_ready && (rc = tables_for(p, ws, s, is_w ? 0 : 1, cur.idx, st))) return rc;
+  SweepParams sp; fill_sweep(p, ws, s, sp);
+  sp.Y = y; sp.Gr = g; sp.bias = p.d.has_bias ? bias : nullptr;
+  sp.order = is_w ? 0 : 1;
+  if ((rc = run_sweep(p, s, sp, st))) return rc;
+  ReduceArgs r{};
+  r.partial = sp.partial; r.n_cand = p.d.eq_n; r.P = 1; r.tiles_m = p.tiles_m; r.tiles_n = p.tiles_o; r.order = sp.order;
+  r.mode = P4V_SG_COLUMN; r.n_keys = p.nsg; r.sums = at<double>(ws, p.o_scores);
+  if ((rc = p4v_reduce_scores(r, st))) return rc;
+  SelectArgs f = select_args(p, ws, cur, score_log);
+  f.n_keys = p.nsg;
+  f.keys_per_group = (is_w && p.d.n_V > 1) ? p.crb_rows / P4V_CG : p.nsg;
+  f.has_next = next != nullptr;
+  if (next) f.next = tables_args(p, ws, step_of(p, *next), next->is_w ? 0 : 1, next->idx);
+  if ((rc = p4v_select_step(f, st))) return rc;
+  return p4v_commit_step(commit_args(p, ws, cur), st);
+}
+
+// The search steps of seq in order.  The scale tables of seq[0] are built first; those of every later step come with
+// the select of the step before it.  The score log gets one [eq_n][groups] table per step.
+int run_steps(const LinPlan& p, void* ws, const std::vector<StepRef>& seq, const float* bias, const float* y, const float* g,
+              float* score_log, cudaStream_t st) {
+  for (size_t i = 0; i < seq.size(); ++i) {
+    int rc = search_step(p, ws, seq[i], i + 1 < seq.size() ? &seq[i + 1] : nullptr, i > 0, bias, y, g, score_log, st);
+    if (rc) return rc;
+    if (score_log) score_log += seq[i].is_w ? (size_t)p.d.eq_n * p.d.n_V : (size_t)p.d.eq_n;
+  }
+  return 0;
+}
+
+void add_steps(std::vector<StepRef>& seq, bool is_w, int begin, int end) {
+  for (int i = begin; i < end; ++i) seq.push_back(StepRef{is_w, i});
 }
 
 // Whole W search of one round in normal-equation form (gram.cu): residual once, then per column block
@@ -559,22 +451,10 @@ int gram_wsearch(const LinPlan& p, void* ws, const float* x, const float* W, con
     ev.sums = at<double>(ws, p.o_scores) + (size_t)p.d.eq_n * p.d.n_V; ev.n_keys = p.d.n_V * p.g_osplit;
     ev.sums2 = at<double>(ws, p.o_scores);
     if ((rc = p4v_gram_eval(ev, st))) return rc;
-    SelectArgs f{};
-    f.sums = ev.sums2; f.n_cand = p.d.eq_n; f.n_keys = p.d.n_V; f.n_groups = p.d.n_V; f.keys_per_group = 1;
-    f.inv_count = 1.0 / ((double)p.d.tokens * (double)p.crb_rows);
-    f.gscale = at<float>(ws, p.o_gscale); f.factors = at<float>(ws, p.o_factors);
-    f.d0 = at<float>(ws, p.o_dW0); f.d = at<float>(ws, p.o_dW); f.d_stride = p.d.n_H; f.d_col = h;
-    f.best = at<int>(ws, p.o_best); f.score_log = score_log; f.d_prev = at<float>(ws, p.o_dprev); f.has_next = 0;
+    SelectArgs f = select_args(p, ws, StepRef{true, h}, score_log);   // ev.sums2: one key per row block
+    f.n_keys = p.d.n_V; f.keys_per_group = 1; f.d_prev = at<float>(ws, p.o_dprev);
     if ((rc = p4v_select_step(f, st))) return rc;
-    const Step& s = p.wsteps[h];
-    CommitArgs c{};
-    c.best = f.best; c.n_groups = p.d.n_V;
-    c.cand = at<uint8_t>(ws, p.o_Wcand); c.cand_tile_bytes = (unsigned long long)P4V_TILE * p.KB_W;
-    c.cand_plane_stride = c.cand_tile_bytes * p.tiles_o;
-    c.cur = at<uint8_t>(ws, p.o_Wcur); c.cur_tile_bytes = c.cand_tile_bytes;
-    c.P = 1; c.tiles = p.tiles_o; c.rows_per_group = p.crb_rows; c.problem_groups = 0;
-    c.segs = at<CommitSeg>(ws, p.o_commits) + s.commit_off; c.nseg = s.ncommit; c.commit_chunks = s.commit_chunks;
-    if ((rc = p4v_commit_step(c, st))) return rc;
+    if ((rc = p4v_commit_step(commit_args(p, ws, StepRef{true, h}), st))) return rc;
     if (score_log) score_log += (size_t)p.d.eq_n * p.d.n_V;
   }
   return 0;
@@ -615,11 +495,7 @@ int begin_impl(const LinPlan& p, const float* x, const float* W, const float* g,
 }  // namespace
 
 extern "C" int p4v_linear_workspace_bytes(const p4v_linear_desc* d, size_t* bytes) {
-  LinPlan p; int rc = build_plan(d, p, true);
-  if (rc) return rc;
-  P4V_REQUIRE(bytes != nullptr, "null output");
-  *bytes = p.total;
-  return 0;
+  return plan_workspace_bytes(build_plan, d, bytes, true);
 }
 
 extern "C" int p4v_linear_score_log_floats(const p4v_linear_desc* d, size_t* n) {
@@ -644,13 +520,9 @@ extern "C" int p4v_linear_search_w(const p4v_linear_desc* d, const float* bias, 
   if (rc) return rc;
   P4V_REQUIRE(raw_out && raw_grad && workspace, "linear_search_w: null pointer");
   P4V_REQUIRE(0 <= h_begin && h_begin <= h_end && h_end <= d->n_H, "linear_search_w: bad block range");
-  for (int h = h_begin; h < h_end; ++h) {
-    StepRef nx{true, h + 1};
-    if ((rc = search_step(p, workspace, StepRef{true, h}, h + 1 < h_end ? &nx : nullptr, h > h_begin, bias, raw_out, raw_grad,
-                          score_log, (cudaStream_t)stream))) return rc;
-    if (score_log) score_log += (size_t)d->eq_n * d->n_V;
-  }
-  return 0;
+  std::vector<StepRef> seq;
+  add_steps(seq, true, h_begin, h_end);
+  return run_steps(p, workspace, seq, bias, raw_out, raw_grad, score_log, (cudaStream_t)stream);
 }
 
 extern "C" int p4v_linear_search_a(const p4v_linear_desc* d, const float* bias, const float* raw_out, const float* raw_grad,
@@ -659,13 +531,9 @@ extern "C" int p4v_linear_search_a(const p4v_linear_desc* d, const float* bias, 
   if (rc) return rc;
   P4V_REQUIRE(raw_out && raw_grad && workspace, "linear_search_a: null pointer");
   P4V_REQUIRE(0 <= a_begin && a_begin <= a_end && a_end <= d->n_a, "linear_search_a: bad chunk range");
-  for (int a = a_begin; a < a_end; ++a) {
-    StepRef nx{false, a + 1};
-    if ((rc = search_step(p, workspace, StepRef{false, a}, a + 1 < a_end ? &nx : nullptr, a > a_begin, bias, raw_out, raw_grad,
-                          score_log, (cudaStream_t)stream))) return rc;
-    if (score_log) score_log += d->eq_n;
-  }
-  return 0;
+  std::vector<StepRef> seq;
+  add_steps(seq, false, a_begin, a_end);
+  return run_steps(p, workspace, seq, bias, raw_out, raw_grad, score_log, (cudaStream_t)stream);
 }
 
 extern "C" int p4v_linear_intervals(const p4v_linear_desc* d, void* workspace, float* w_interval, float* a_interval, void* stream) {
@@ -688,27 +556,21 @@ extern "C" int p4v_linear_calibrate(const p4v_linear_desc* d, const float* x, co
   cudaStream_t st = (cudaStream_t)stream;
   if ((rc = begin_impl(p, x, weight, raw_grad, workspace, st))) return rc;
   if (p.gram) {
+    std::vector<StepRef> xseq;
+    add_steps(xseq, false, 0, d->n_a);
     for (int e = 0; e < d->search_round; ++e) {
       if ((rc = gram_wsearch(p, workspace, x, weight, bias, raw_out, raw_grad, 0, d->n_H, score_log, st))) return rc;
       if (score_log) score_log += (size_t)d->n_H * d->eq_n * d->n_V;
-      for (int a = 0; a < d->n_a; ++a) {
-        StepRef nx{false, a + 1};
-        if ((rc = search_step(p, workspace, StepRef{false, a}, a + 1 < d->n_a ? &nx : nullptr, a > 0, bias, raw_out, raw_grad,
-                              score_log, st))) return rc;
-        if (score_log) score_log += d->eq_n;
-      }
+      if ((rc = run_steps(p, workspace, xseq, bias, raw_out, raw_grad, score_log, st))) return rc;
+      if (score_log) score_log += (size_t)d->n_a * d->eq_n;
     }
-  } else {
+  } else {   // one sequence over all rounds: every select prepares the next step's tables, across W/X boundaries too
     std::vector<StepRef> seq;
     for (int e = 0; e < d->search_round; ++e) {
-      for (int h = 0; h < d->n_H; ++h) seq.push_back(StepRef{true, h});
-      for (int a = 0; a < d->n_a; ++a) seq.push_back(StepRef{false, a});
+      add_steps(seq, true, 0, d->n_H);
+      add_steps(seq, false, 0, d->n_a);
     }
-    for (size_t i = 0; i < seq.size(); ++i) {
-      if ((rc = search_step(p, workspace, seq[i], i + 1 < seq.size() ? &seq[i + 1] : nullptr, i > 0, bias, raw_out, raw_grad,
-                            score_log, st))) return rc;
-      if (score_log) score_log += seq[i].is_w ? (size_t)d->eq_n * d->n_V : (size_t)d->eq_n;
-    }
+    if ((rc = run_steps(p, workspace, seq, bias, raw_out, raw_grad, score_log, st))) return rc;
   }
   P4V_CUDA_OK(cudaMemcpyAsync(w_interval, at<float>(workspace, p.o_dW), (size_t)d->n_V * d->n_H * 4, cudaMemcpyDeviceToDevice, st));
   P4V_CUDA_OK(cudaMemcpyAsync(a_interval, at<float>(workspace, p.o_dX), (size_t)d->n_a * 4, cudaMemcpyDeviceToDevice, st));
@@ -716,11 +578,7 @@ extern "C" int p4v_linear_calibrate(const p4v_linear_desc* d, const float* x, co
 }
 
 extern "C" int p4v_linear_quant_forward_workspace_bytes(const p4v_linear_desc* d, size_t* bytes) {
-  LinPlan p; int rc = build_plan(d, p, false);
-  if (rc) return rc;
-  P4V_REQUIRE(bytes != nullptr, "null output");
-  *bytes = p.total;
-  return 0;
+  return plan_workspace_bytes(build_plan, d, bytes, false);
 }
 
 extern "C" int p4v_linear_quant_forward(const p4v_linear_desc* d, const float* x, const float* weight, const float* bias,

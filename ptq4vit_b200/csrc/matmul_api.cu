@@ -5,15 +5,10 @@
 #include <vector>
 
 #include "../../include/ptq4vit_b200.h"
+#include "plan.cuh"
 #include "prep.cuh"
 
-void p4v_count_launch();
-int p4v_run_sweep(const SweepParams& sp, const P4VJob* host_jobs, int kernel, cudaStream_t st);
-
 namespace {
-
-inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
-template <class T> T* at(void* ws, size_t off) { return reinterpret_cast<T*>(static_cast<uint8_t*>(ws) + off); }
 
 struct MStep { int job_off, nfj, ncj, nfg, ncg, meta_fix, meta_cand; };
 
@@ -35,17 +30,6 @@ struct MMPlan {
       o_Bcand, o_Ascand, o_Bsplit, total;
 };
 
-void push_jobs(MMPlan& p, int r_off, int c_off, int kb, uint8_t src, int group, bool first, bool last, int& n) {
-  for (int b = 0; b < kb; b += P4V_JOB_KB) {
-    P4VJob j{};
-    const int len = std::min(P4V_JOB_KB, kb - b);
-    j.r_off = (uint32_t)(r_off + b) * P4V_TILE; j.c_off = (uint32_t)(c_off + b) * P4V_TILE; j.kb = (uint8_t)len;
-    j.flags = src | ((first && b == 0) ? P4V_JOB_FIRST : 0) | ((last && b + len >= kb) ? P4V_JOB_LAST : 0);
-    j.group = (uint8_t)group;
-    p.jobs.push_back(j); ++n;
-  }
-}
-
 int build_plan(const p4v_matmul_desc* d, MMPlan& p, bool with_search) {
   P4V_REQUIRE(d != nullptr, "null desc");
   p.d = *d;
@@ -56,9 +40,7 @@ int build_plan(const p4v_matmul_desc* d, MMPlan& p, bool with_search) {
   p.H = d->heads; p.P = d->batch * d->heads; p.S1 = d->S1; p.S2 = d->S2; p.S3 = d->S3;
   p.A_qmax = 1 << (d->A_bit - 1); p.B_qmax = 1 << (d->B_bit - 1);
   p.tiles_m = p4v_cdiv(p.S1, P4V_TILE); p.tiles_n = p4v_cdiv(p.S3, P4V_TILE);
-  if (d->operand == P4V_OPERAND_INT8) p.i8 = true;
-  else if (d->operand == P4V_OPERAND_BF16) p.i8 = false;
-  else p.i8 = p.S2 >= 64;
+  p.i8 = use_int8(d->operand, p.S2);
   p.ew = p.i8 ? 1 : 2;
   p.kb = (int)align_up((size_t)p.S2 * p.ew, 32);
   p.kb16 = (int)align_up((size_t)p.S2 * 2, 32);
@@ -78,8 +60,7 @@ int build_plan(const p4v_matmul_desc* d, MMPlan& p, bool with_search) {
   }
   p.segB.push_back(P4VSeg{0, p.S2, 0, 0, 0.f, (float)-p.B_qmax, (float)(p.B_qmax - 1), 0, 0.f, 0, 0});
 
-  p.factors.resize(d->eq_n + 1);
-  for (int i = 0; i <= d->eq_n; ++i) p.factors[i] = (float)(d->eq_alpha + i * (d->eq_beta - d->eq_alpha) / d->eq_n);
+  p.factors = candidate_factors(d->eq_alpha, d->eq_beta, d->eq_n);
   p.n_split = 20;                                         // matmul.py:636
   p.split_factors.resize(p.n_split);
   for (int i = 0; i < p.n_split; ++i) p.split_factors[i] = (float)(1.0 / (double)(1u << i));
@@ -90,90 +71,80 @@ int build_plan(const p4v_matmul_desc* d, MMPlan& p, bool with_search) {
   if (with_search) {
     if (!p.sos) {   // A step: candidates on the row operand
       begin(p.stepA); p.stepA.meta_cand = (int)p.metas.size();
-      push_jobs(p, 0, 0, p.kb, P4V_JOB_RCAND, 0, true, true, p.stepA.ncj);
+      push_jobs(p.jobs, 0, 0, p.kb, P4V_JOB_RCAND, 0, true, true, p.stepA.ncj);
       p.metas.push_back(GroupMeta{0, 0, 0, 0}); p.stepA.ncg = 1;
     } else {        // split search: (hi,lo)_c x exact 3-term bf16 split of the unquantised B
       begin(p.stepS); p.stepS.meta_cand = (int)p.metas.size();
       for (int part = 0; part < 2; ++part) {
         for (int t = 0; t < 3; ++t)
-          push_jobs(p, part * p.kb16, t * p.kb16, p.kb16, P4V_JOB_RCAND, part, t == 0, t == 2, p.stepS.ncj);
+          push_jobs(p.jobs, part * p.kb16, t * p.kb16, p.kb16, P4V_JOB_RCAND, part, t == 0, t == 2, p.stepS.ncj);
         p.metas.push_back(GroupMeta{0, 0, 0, 0});        // both parts use aux[0] = 1/(qmax-1); lo also the candidate split
         ++p.stepS.ncg;
       }
     }
     begin(p.stepB); p.stepB.meta_cand = (int)p.metas.size();
     if (!p.sos) {
-      push_jobs(p, 0, 0, p.kb, P4V_JOB_CCAND, 0, true, true, p.stepB.ncj);
+      push_jobs(p.jobs, 0, 0, p.kb, P4V_JOB_CCAND, 0, true, true, p.stepB.ncj);
       p.metas.push_back(GroupMeta{0, 0, 0, 0}); p.stepB.ncg = 1;
     } else {
       for (int part = 0; part < 2; ++part) {
-        push_jobs(p, part * p.kb, 0, p.kb, P4V_JOB_CCAND, part, true, true, p.stepB.ncj);
+        push_jobs(p.jobs, part * p.kb, 0, p.kb, P4V_JOB_CCAND, part, true, true, p.stepB.ncj);
         p.metas.push_back(GroupMeta{0, (short)part, 0, 0}); ++p.stepB.ncg;     // aux[0] = 1/(qmax-1), aux[1] = A_interval
       }
     }
-    {   // the row operand (A) of the B step is the same for every candidate: keep it resident when it is small
-      uint32_t total = 0, off = 0;
-      for (int j = 0; j < p.stepB.ncj; ++j) total += (uint32_t)p.jobs[p.stepB.job_off + j].kb * P4V_TILE;
-      if (total <= 60 * 1024)
-        for (int j = 0; j < p.stepB.ncj; ++j) {
-          P4VJob& jb = p.jobs[p.stepB.job_off + j];
-          jb.flags |= P4V_JOB_RRES; jb.res_off = off; off += (uint32_t)jb.kb * P4V_TILE;
-        }
-    }
+    mark_resident(p.jobs, p.stepB.job_off + p.stepB.nfj, p.stepB.ncj);   // the B step's row operand (A) is candidate independent
   }
   begin(p.fwd);
-  if (!p.sos) { push_jobs(p, 0, 0, p.kb, 0, 0, true, true, p.fwd.nfj); p.metas.push_back(GroupMeta{0, 0, 0, 0}); p.fwd.nfg = 1; }
+  if (!p.sos) { push_jobs(p.jobs, 0, 0, p.kb, 0, 0, true, true, p.fwd.nfj); p.metas.push_back(GroupMeta{0, 0, 0, 0}); p.fwd.nfg = 1; }
   else for (int part = 0; part < 2; ++part) {
-    push_jobs(p, part * p.kb, 0, p.kb, 0, part, true, true, p.fwd.nfj);
+    push_jobs(p.jobs, part * p.kb, 0, p.kb, 0, part, true, true, p.fwd.nfj);
     p.metas.push_back(GroupMeta{0, (short)part, 0, 0}); ++p.fwd.nfg;
   }
   p.fwd.meta_cand = (int)p.metas.size();
   P4V_REQUIRE((int)p.jobs.size() <= 4 * P4V_MAX_JOBS && p.stepS.ncj <= P4V_MAX_JOBS && p.stepB.ncj <= P4V_MAX_JOBS &&
               p.stepA.ncj <= P4V_MAX_JOBS && p.fwd.nfj <= P4V_MAX_JOBS, "matmul: S2 too large");
 
-  size_t o = 0;
-  auto take = [&](size_t bytes) { size_t r = o; o = align_up(o + bytes, 256); return r; };
+  Carver w;
   const int n_c = std::max(d->eq_n, p.n_split);
-  p.o_factors = take((d->eq_n + 1) * 4); p.o_sfactors = take(p.n_split * 4);
-  p.o_keys = take((2 * p.H + 1) * 4);
-  p.o_dA0 = take(p.H * 4); p.o_dA = take(p.H * 4); p.o_dB0 = take(p.H * 4); p.o_dB = take(p.H * 4);
-  p.o_ones = take(p.H * 4); p.o_aux = take(2 * 4); p.o_split = take(4); p.o_gscale = take(4);
-  p.o_scores = take((size_t)n_c * p.H * 8); p.o_best = take(p.H * 4);
-  p.o_fix = take((size_t)2 * p.H * 4); p.o_candA = take((size_t)n_c * p.H * 4); p.o_candB = take((size_t)2 * p.H * 4);
-  p.o_jobs = take(p.jobs.size() * sizeof(P4VJob)); p.o_metas = take(p.metas.size() * sizeof(GroupMeta));
-  p.o_segA = take(p.segA.size() * sizeof(P4VSeg)); p.o_segB = take(p.segB.size() * sizeof(P4VSeg));
-  p.o_segAs = take(std::max<size_t>(1, p.segAs.size()) * sizeof(P4VSeg));
-  p.o_segBs = take(std::max<size_t>(1, p.segBs.size()) * sizeof(P4VSeg));
+  p.o_factors = w.take((d->eq_n + 1) * 4); p.o_sfactors = w.take(p.n_split * 4);
+  p.o_keys = w.take((2 * p.H + 1) * 4);
+  p.o_dA0 = w.take(p.H * 4); p.o_dA = w.take(p.H * 4); p.o_dB0 = w.take(p.H * 4); p.o_dB = w.take(p.H * 4);
+  p.o_ones = w.take(p.H * 4); p.o_aux = w.take(2 * 4); p.o_split = w.take(4); p.o_gscale = w.take(4);
+  p.o_scores = w.take((size_t)n_c * p.H * 8); p.o_best = w.take(p.H * 4);
+  p.o_fix = w.take((size_t)2 * p.H * 4); p.o_candA = w.take((size_t)n_c * p.H * 4); p.o_candB = w.take((size_t)2 * p.H * 4);
+  p.o_jobs = w.take(p.jobs.size() * sizeof(P4VJob)); p.o_metas = w.take(p.metas.size() * sizeof(GroupMeta));
+  p.o_segA = w.take(p.segA.size() * sizeof(P4VSeg)); p.o_segB = w.take(p.segB.size() * sizeof(P4VSeg));
+  p.o_segAs = w.take(std::max<size_t>(1, p.segAs.size()) * sizeof(P4VSeg));
+  p.o_segBs = w.take(std::max<size_t>(1, p.segBs.size()) * sizeof(P4VSeg));
   const size_t tilesA = (size_t)p.P * p.tiles_m, tilesB = (size_t)p.P * p.tiles_n;
-  p.o_partial = take(with_search ? tilesA * p.tiles_n * n_c * 32 * 4 : 4);
-  p.o_Acur = take(tilesA * P4V_TILE * p.KB_A);
-  p.o_Bcur = take(tilesB * P4V_TILE * p.KB_B);
-  p.o_Acand = take(with_search && !p.sos ? (size_t)d->eq_n * tilesA * P4V_TILE * p.KB_A : 4);
-  p.o_Bcand = take(with_search ? (size_t)d->eq_n * tilesB * P4V_TILE * p.KB_B : 4);
-  p.o_Ascand = take(with_search && p.sos ? (size_t)p.n_split * tilesA * P4V_TILE * p.KB_As : 4);
-  p.o_Bsplit = take(with_search && p.sos ? tilesB * P4V_TILE * p.KB_Bs : 4);
-  p.total = o;
+  p.o_partial = w.take(with_search ? tilesA * p.tiles_n * n_c * 32 * 4 : 4);
+  p.o_Acur = w.take(tilesA * P4V_TILE * p.KB_A);
+  p.o_Bcur = w.take(tilesB * P4V_TILE * p.KB_B);
+  p.o_Acand = w.take(with_search && !p.sos ? (size_t)d->eq_n * tilesA * P4V_TILE * p.KB_A : 4);
+  p.o_Bcand = w.take(with_search ? (size_t)d->eq_n * tilesB * P4V_TILE * p.KB_B : 4);
+  p.o_Ascand = w.take(with_search && p.sos ? (size_t)p.n_split * tilesA * P4V_TILE * p.KB_As : 4);
+  p.o_Bsplit = w.take(with_search && p.sos ? tilesB * P4V_TILE * p.KB_Bs : 4);
+  p.total = w.total;
   return 0;
 }
 
-int upload(const MMPlan& p, void* ws, cudaStream_t st) {
-  P4V_CUDA_OK(cudaMemcpyAsync(at<void>(ws, p.o_factors), p.factors.data(), p.factors.size() * 4, cudaMemcpyHostToDevice, st));
-  P4V_CUDA_OK(cudaMemcpyAsync(at<void>(ws, p.o_sfactors), p.split_factors.data(), p.split_factors.size() * 4, cudaMemcpyHostToDevice, st));
-  P4V_CUDA_OK(cudaMemcpyAsync(at<void>(ws, p.o_jobs), p.jobs.data(), p.jobs.size() * sizeof(P4VJob), cudaMemcpyHostToDevice, st));
-  P4V_CUDA_OK(cudaMemcpyAsync(at<void>(ws, p.o_metas), p.metas.data(), p.metas.size() * sizeof(GroupMeta), cudaMemcpyHostToDevice, st));
-  P4V_CUDA_OK(cudaMemcpyAsync(at<void>(ws, p.o_segA), p.segA.data(), p.segA.size() * sizeof(P4VSeg), cudaMemcpyHostToDevice, st));
-  P4V_CUDA_OK(cudaMemcpyAsync(at<void>(ws, p.o_segB), p.segB.data(), p.segB.size() * sizeof(P4VSeg), cudaMemcpyHostToDevice, st));
-  if (!p.segAs.empty()) P4V_CUDA_OK(cudaMemcpyAsync(at<void>(ws, p.o_segAs), p.segAs.data(), p.segAs.size() * sizeof(P4VSeg), cudaMemcpyHostToDevice, st));
-  if (!p.segBs.empty()) P4V_CUDA_OK(cudaMemcpyAsync(at<void>(ws, p.o_segBs), p.segBs.data(), p.segBs.size() * sizeof(P4VSeg), cudaMemcpyHostToDevice, st));
-  std::vector<float> ones(p.H, 1.f);
-  P4V_CUDA_OK(cudaMemcpyAsync(at<void>(ws, p.o_ones), ones.data(), p.H * 4, cudaMemcpyHostToDevice, st));
+int upload_tables(const MMPlan& p, void* ws, cudaStream_t st) {
+  int rc;
+  if ((rc = upload(ws, p.o_factors, p.factors, st)) || (rc = upload(ws, p.o_sfactors, p.split_factors, st)) ||
+      (rc = upload(ws, p.o_jobs, p.jobs, st)) || (rc = upload(ws, p.o_metas, p.metas, st)) ||
+      (rc = upload(ws, p.o_segA, p.segA, st)) || (rc = upload(ws, p.o_segB, p.segB, st)) ||
+      (rc = upload(ws, p.o_segAs, p.segAs, st)) || (rc = upload(ws, p.o_segBs, p.segBs, st)) ||
+      (rc = upload(ws, p.o_ones, std::vector<float>(p.H, 1.f), st))) return rc;
   return 0;
 }
 
-// which: 0 Acur, 1 Acand, 2 Bcur, 3 Bcand, 4 A split-search candidates (bf16), 5 B exact split (bf16)
-int quant(const MMPlan& p, void* ws, int which, const float* src, cudaStream_t st) {
+// The operand images quant() writes: the current A / B images, their candidate planes, and the two bf16 images of the
+// split search (A's split candidates, the exact three-term split of B).
+enum Image { A_CUR, A_CAND, B_CUR, B_CAND, A_SPLIT_CAND, B_SPLIT };
+
+int quant(const MMPlan& p, void* ws, Image which, const float* src, cudaStream_t st) {
   QuantImageArgs q{};
-  const bool isA = which == 0 || which == 1 || which == 4;
+  const bool isA = which == A_CUR || which == A_CAND || which == A_SPLIT_CAND;
   q.src = src; q.P = p.P; q.prob_stride = isA ? (long long)p.S1 * p.S2 : (long long)p.S2 * p.S3;
   q.src_transposed = isA ? 0 : 1; q.ld = isA ? p.S2 : p.S3;
   q.rows = isA ? p.S1 : p.S3; q.tiles = isA ? p.tiles_m : p.tiles_n;
@@ -181,15 +152,15 @@ int quant(const MMPlan& p, void* ws, int which, const float* src, cudaStream_t s
   q.is_int8 = p.i8; q.n_planes = 1; q.factors = nullptr; q.split = at<float>(ws, p.o_split);
   int KB = 0;
   switch (which) {
-    case 0: q.dst = at<uint8_t>(ws, p.o_Acur); KB = p.KB_A; q.delta = at<float>(ws, p.o_dA); q.segs = at<P4VSeg>(ws, p.o_segA); q.nseg = (int)p.segA.size(); break;
-    case 1: q.dst = at<uint8_t>(ws, p.o_Acand); KB = p.KB_A; q.delta = at<float>(ws, p.o_dA0); q.segs = at<P4VSeg>(ws, p.o_segA); q.nseg = (int)p.segA.size();
+    case A_CUR: q.dst = at<uint8_t>(ws, p.o_Acur); KB = p.KB_A; q.delta = at<float>(ws, p.o_dA); q.segs = at<P4VSeg>(ws, p.o_segA); q.nseg = (int)p.segA.size(); break;
+    case A_CAND: q.dst = at<uint8_t>(ws, p.o_Acand); KB = p.KB_A; q.delta = at<float>(ws, p.o_dA0); q.segs = at<P4VSeg>(ws, p.o_segA); q.nseg = (int)p.segA.size();
             q.n_planes = p.d.eq_n; q.factors = at<float>(ws, p.o_factors); break;
-    case 2: q.dst = at<uint8_t>(ws, p.o_Bcur); KB = p.KB_B; q.delta = at<float>(ws, p.o_dB); q.segs = at<P4VSeg>(ws, p.o_segB); q.nseg = 1; break;
-    case 3: q.dst = at<uint8_t>(ws, p.o_Bcand); KB = p.KB_B; q.delta = at<float>(ws, p.o_dB0); q.segs = at<P4VSeg>(ws, p.o_segB); q.nseg = 1;
+    case B_CUR: q.dst = at<uint8_t>(ws, p.o_Bcur); KB = p.KB_B; q.delta = at<float>(ws, p.o_dB); q.segs = at<P4VSeg>(ws, p.o_segB); q.nseg = 1; break;
+    case B_CAND: q.dst = at<uint8_t>(ws, p.o_Bcand); KB = p.KB_B; q.delta = at<float>(ws, p.o_dB0); q.segs = at<P4VSeg>(ws, p.o_segB); q.nseg = 1;
             q.n_planes = p.d.eq_n; q.factors = at<float>(ws, p.o_factors); break;
-    case 4: q.dst = at<uint8_t>(ws, p.o_Ascand); KB = p.KB_As; q.delta = at<float>(ws, p.o_dA0); q.segs = at<P4VSeg>(ws, p.o_segAs); q.nseg = 2;
+    case A_SPLIT_CAND: q.dst = at<uint8_t>(ws, p.o_Ascand); KB = p.KB_As; q.delta = at<float>(ws, p.o_dA0); q.segs = at<P4VSeg>(ws, p.o_segAs); q.nseg = 2;
             q.n_planes = p.n_split; q.factors = at<float>(ws, p.o_sfactors); q.is_int8 = 0; break;
-    default: q.dst = at<uint8_t>(ws, p.o_Bsplit); KB = p.KB_Bs; q.delta = at<float>(ws, p.o_dB0); q.segs = at<P4VSeg>(ws, p.o_segBs); q.nseg = 3; q.is_int8 = 0; break;
+    case B_SPLIT: q.dst = at<uint8_t>(ws, p.o_Bsplit); KB = p.KB_Bs; q.delta = at<float>(ws, p.o_dB0); q.segs = at<P4VSeg>(ws, p.o_segBs); q.nseg = 3; q.is_int8 = 0; break;
   }
   q.tile_bytes = (unsigned long long)P4V_TILE * KB;
   q.plane_stride = q.tile_bytes * q.tiles * p.P;
@@ -263,7 +234,7 @@ int search_A(const MMPlan& p, void* ws, const float* A, const float* Y, const fl
   if ((rc = run_sweep(p, p.stepA, sp, st))) return rc;
   if ((rc = reduce_finish(p, ws, sp, p.d.eq_n, p.H, 1.0 / ((double)p.S1 * p.S3), at<float>(ws, p.o_factors),
                           at<float>(ws, p.o_dA0), at<float>(ws, p.o_dA), log, st))) return rc;
-  return quant(p, ws, 0, A, st);
+  return quant(p, ws, A_CUR, A, st);
 }
 
 int search_B(const MMPlan& p, void* ws, const float* B, const float* Y, const float* G, float* log, cudaStream_t st) {
@@ -275,7 +246,7 @@ int search_B(const MMPlan& p, void* ws, const float* B, const float* Y, const fl
   if ((rc = run_sweep(p, p.stepB, sp, st))) return rc;
   if ((rc = reduce_finish(p, ws, sp, p.d.eq_n, p.H, 1.0 / ((double)p.S1 * p.S3), at<float>(ws, p.o_factors),
                           at<float>(ws, p.o_dB0), at<float>(ws, p.o_dB), log, st))) return rc;
-  return quant(p, ws, 2, B, st);
+  return quant(p, ws, B_CUR, B, st);
 }
 
 int search_split(const MMPlan& p, void* ws, const float* A, const float* Y, const float* G, float* log, cudaStream_t st) {
@@ -295,12 +266,12 @@ int search_split(const MMPlan& p, void* ws, const float* A, const float* Y, cons
   sos_aux_kernel<<<1, 1, 0, st>>>(at<float>(ws, p.o_split), (float)(p.A_qmax - 1), at<float>(ws, p.o_aux), nullptr);
   p4v_count_launch();
   P4V_CUDA_OK(cudaGetLastError());
-  return quant(p, ws, 0, A, st);
+  return quant(p, ws, A_CUR, A, st);
 }
 
 int begin(const MMPlan& p, void* ws, const float* A, const float* B, const float* G, cudaStream_t st) {
   int rc;
-  if ((rc = upload(p, ws, st))) return rc;
+  if ((rc = upload_tables(p, ws, st))) return rc;
   int* keys = at<int>(ws, p.o_keys);
   if ((rc = p4v_keys_reset(keys, 2 * p.H + 1, st))) return rc;
   if ((rc = p4v_group_absmax(A, (long long)p.S1 * p.S2, p.P, p.H, keys, st))) return rc;
@@ -317,25 +288,21 @@ int begin(const MMPlan& p, void* ws, const float* A, const float* B, const float
     set_scalar_kernel<<<1, 1, 0, st>>>(at<float>(ws, p.o_split), 0.01f);       // matmul.py:354-355 (dead: overwritten by the first search)
     sos_aux_kernel<<<1, 1, 0, st>>>(at<float>(ws, p.o_split), (float)(p.A_qmax - 1), at<float>(ws, p.o_aux), nullptr);
     P4V_CUDA_OK(cudaGetLastError());
-    if ((rc = quant(p, ws, 4, A, st))) return rc;
-    if ((rc = quant(p, ws, 5, B, st))) return rc;
+    if ((rc = quant(p, ws, A_SPLIT_CAND, A, st))) return rc;
+    if ((rc = quant(p, ws, B_SPLIT, B, st))) return rc;
   } else {
-    if ((rc = quant(p, ws, 1, A, st))) return rc;
+    if ((rc = quant(p, ws, A_CAND, A, st))) return rc;
   }
-  if ((rc = quant(p, ws, 0, A, st))) return rc;
-  if ((rc = quant(p, ws, 2, B, st))) return rc;
-  if ((rc = quant(p, ws, 3, B, st))) return rc;
+  if ((rc = quant(p, ws, A_CUR, A, st))) return rc;
+  if ((rc = quant(p, ws, B_CUR, B, st))) return rc;
+  if ((rc = quant(p, ws, B_CAND, B, st))) return rc;
   return 0;
 }
 
 }  // namespace
 
 extern "C" int p4v_matmul_workspace_bytes(const p4v_matmul_desc* d, size_t* bytes) {
-  MMPlan p; int rc = build_plan(d, p, true);
-  if (rc) return rc;
-  P4V_REQUIRE(bytes != nullptr, "null output");
-  *bytes = p.total;
-  return 0;
+  return plan_workspace_bytes(build_plan, d, bytes, true);
 }
 
 extern "C" int p4v_matmul_score_log_floats(const p4v_matmul_desc* d, size_t* n) {
@@ -376,11 +343,7 @@ extern "C" int p4v_matmul_calibrate(const p4v_matmul_desc* d, const float* A, co
 }
 
 extern "C" int p4v_matmul_quant_forward_workspace_bytes(const p4v_matmul_desc* d, size_t* bytes) {
-  MMPlan p; int rc = build_plan(d, p, false);
-  if (rc) return rc;
-  P4V_REQUIRE(bytes != nullptr, "null output");
-  *bytes = p.total;
-  return 0;
+  return plan_workspace_bytes(build_plan, d, bytes, false);
 }
 
 extern "C" int p4v_matmul_quant_forward(const p4v_matmul_desc* d, const float* A, const float* B, const float* A_interval,
@@ -392,7 +355,7 @@ extern "C" int p4v_matmul_quant_forward(const p4v_matmul_desc* d, const float* A
   P4V_REQUIRE(!p.sos || split, "matmul_quant_forward: sos needs split");
   P4V_REQUIRE(workspace_bytes >= p.total, "matmul_quant_forward: workspace too small (%zu < %zu)", workspace_bytes, p.total);
   cudaStream_t st = (cudaStream_t)stream;
-  if ((rc = upload(p, workspace, st))) return rc;
+  if ((rc = upload_tables(p, workspace, st))) return rc;
   P4V_CUDA_OK(cudaMemcpyAsync(at<float>(workspace, p.o_dB), B_interval, (size_t)p.H * 4, cudaMemcpyDeviceToDevice, st));
   if (p.sos) {
     P4V_CUDA_OK(cudaMemcpyAsync(at<float>(workspace, p.o_split), split, 4, cudaMemcpyDeviceToDevice, st));
@@ -401,8 +364,8 @@ extern "C" int p4v_matmul_quant_forward(const p4v_matmul_desc* d, const float* A
   } else {
     P4V_CUDA_OK(cudaMemcpyAsync(at<float>(workspace, p.o_dA), A_interval, (size_t)p.H * 4, cudaMemcpyDeviceToDevice, st));
   }
-  if ((rc = quant(p, workspace, 0, A, st))) return rc;
-  if ((rc = quant(p, workspace, 2, B, st))) return rc;
+  if ((rc = quant(p, workspace, A_CUR, A, st))) return rc;
+  if ((rc = quant(p, workspace, B_CUR, B, st))) return rc;
   // fixed scale per head: plain dA*dB ; sos: dB * aux[part]
   if ((rc = tables(p, workspace, p.fwd, p.sos ? 3 : 2, at<float>(workspace, p.o_dB0),
                    p.sos ? at<float>(workspace, p.o_dB) : at<float>(workspace, p.o_dA),

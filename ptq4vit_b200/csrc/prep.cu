@@ -3,8 +3,6 @@
 #include <math.h>
 #include <stdlib.h>
 
-void p4v_count_launch();
-
 namespace {
 
 // order-preserving float <-> int key (so that atomicMax on ints is max on floats)

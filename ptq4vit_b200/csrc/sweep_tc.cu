@@ -252,33 +252,22 @@ __device__ __forceinline__ f32x2 mul2(f32x2 a, f32x2 b) { f32x2 d; asm("mul.rn.f
 // against the running residual.
 //   kScore == false:  r -= s * acc                        (fixed segments / non-final candidate segments)
 //   kScore == true :  p = sum (g * (r - s*acc))^2          (final candidate segment; r is not modified)
-template <bool kInt8, bool kScore, bool kPacked, int OFF>
+template <bool kInt8, bool kScore, int OFF>
 __device__ __forceinline__ void consume16(const uint32_t (&a)[16], float (&r)[64], const float (&g)[64], const float s, float& p) {
-  if constexpr (kPacked) {
-    f32x2 q0 = 0ull, q1 = 0ull;
-    const f32x2 ns = pack2(-s, -s);
+  f32x2 q0 = 0ull, q1 = 0ull;
+  const f32x2 ns = pack2(-s, -s);
 #pragma unroll
-    for (int j = 0; j < 16; j += 2) {
-      const f32x2 f = pack2(acc_to_float<kInt8>(a[j]), acc_to_float<kInt8>(a[j + 1]));
-      const f32x2 d = fma2(ns, f, pack2(r[OFF + j], r[OFF + j + 1]));
-      if constexpr (kScore) {
-        const f32x2 w = mul2(pack2(g[OFF + j], g[OFF + j + 1]), d);
-        if (j & 2) q1 = fma2(w, w, q1); else q0 = fma2(w, w, q0);
-      } else {
-        unpack2(d, r[OFF + j], r[OFF + j + 1]);
-      }
+  for (int j = 0; j < 16; j += 2) {
+    const f32x2 f = pack2(acc_to_float<kInt8>(a[j]), acc_to_float<kInt8>(a[j + 1]));
+    const f32x2 d = fma2(ns, f, pack2(r[OFF + j], r[OFF + j + 1]));
+    if constexpr (kScore) {
+      const f32x2 w = mul2(pack2(g[OFF + j], g[OFF + j + 1]), d);
+      if (j & 2) q1 = fma2(w, w, q1); else q0 = fma2(w, w, q0);
+    } else {
+      unpack2(d, r[OFF + j], r[OFF + j + 1]);
     }
-    if constexpr (kScore) { float x0, y0, x1, y1; unpack2(q0, x0, y0); unpack2(q1, x1, y1); p = (x0 + y0) + (x1 + y1); }
-  } else {
-    float q0 = 0.f, q1 = 0.f;
-#pragma unroll
-    for (int j = 0; j < 16; ++j) {
-      const float d = fmaf(-s, acc_to_float<kInt8>(a[j]), r[OFF + j]);
-      if constexpr (kScore) { const float w = g[OFF + j] * d; if (j & 1) q1 = fmaf(w, w, q1); else q0 = fmaf(w, w, q0); }
-      else r[OFF + j] = d;
-    }
-    if constexpr (kScore) p = q0 + q1;
   }
+  if constexpr (kScore) { float x0, y0, x1, y1; unpack2(q0, x0, y0); unpack2(q1, x1, y1); p = (x0 + y0) + (x1 + y1); }
 }
 
 // Reduce 4 per-lane values over the 32 lanes (= rows) of the warp, fixed order: lane 8*k ends up with the total of value k.
@@ -314,7 +303,7 @@ __device__ __forceinline__ void acc_begin(SmemCtl& S, AccRing& ring, uint32_t tb
 
 // One accumulator = four 16-column quarters, double buffered in a0/a1: the TMEM load of the next quarter is in flight
 // while the CUDA cores work on the current one; the slot returns to the MMA warp once its last quarter is in registers.
-template <bool kInt8, bool kScore, bool kPacked>
+template <bool kInt8, bool kScore>
 __device__ __forceinline__ void acc_step(SmemCtl& S, AccRing& ring, uint32_t tbase, int lane, uint32_t (&a0)[16],
                                          uint32_t (&a1)[16], float (&r)[64], const float (&g)[64], const float4 sc,
                                          float (&p)[4], const bool has_next, const bool skip_math = false) {
@@ -335,13 +324,13 @@ __device__ __forceinline__ void acc_step(SmemCtl& S, AccRing& ring, uint32_t tba
   bool next_ready = true;
   if (has_next) next_ready = mbar_try(next_bar, nphase);
   tmem_ld16(t0 + 16, a1);
-  consume16<kInt8, kScore, kPacked, 0>(a0, r, g, sc.x, p[0]);
+  consume16<kInt8, kScore, 0>(a0, r, g, sc.x, p[0]);
   tmem_wait_ld();
   tmem_ld16(t0 + 32, a0);
-  consume16<kInt8, kScore, kPacked, 16>(a1, r, g, sc.y, p[1]);
+  consume16<kInt8, kScore, 16>(a1, r, g, sc.y, p[1]);
   tmem_wait_ld();
   tmem_ld16(t0 + 48, a1);
-  consume16<kInt8, kScore, kPacked, 32>(a0, r, g, sc.z, p[2]);
+  consume16<kInt8, kScore, 32>(a0, r, g, sc.z, p[2]);
   tmem_wait_ld();
   tc_fence_before();
   __syncwarp();
@@ -352,7 +341,7 @@ __device__ __forceinline__ void acc_step(SmemCtl& S, AccRing& ring, uint32_t tba
     tc_fence_after();
     tmem_ld16(tbase + nslot * kAccCols, a0);
   }
-  consume16<kInt8, kScore, kPacked, 48>(a1, r, g, sc.w, p[3]);
+  consume16<kInt8, kScore, 48>(a1, r, g, sc.w, p[3]);
   if (has_next) tmem_wait_ld();
 }
 
@@ -373,20 +362,15 @@ __device__ __forceinline__ void tmem_ld32u(uint32_t taddr, uint32_t (&v)[32]) {
       : "r"(taddr));
 }
 // gp: this thread's row of the parked gradient tile, [column quad][128 rows] float4 (quad stride = 128 float4)
-template <bool kInt8, bool kScore, bool kPacked, int OFF>
+template <bool kInt8, bool kScore, int OFF>
 __device__ __forceinline__ void consume32(const uint32_t (&a)[32], float (&r)[64], const float4* gp, const float s0,
                                           const float s1, float& p0, float& p1) {
   if constexpr (!kScore) {
 #pragma unroll
     for (int j = 0; j < 32; j += 2) {
       const float s = j < 16 ? s0 : s1;
-      if constexpr (kPacked) {
-        const f32x2 d = fma2(pack2(-s, -s), pack2(acc_to_float<kInt8>(a[j]), acc_to_float<kInt8>(a[j + 1])), pack2(r[OFF + j], r[OFF + j + 1]));
-        unpack2(d, r[OFF + j], r[OFF + j + 1]);
-      } else {
-        r[OFF + j] = fmaf(-s, acc_to_float<kInt8>(a[j]), r[OFF + j]);
-        r[OFF + j + 1] = fmaf(-s, acc_to_float<kInt8>(a[j + 1]), r[OFF + j + 1]);
-      }
+      const f32x2 d = fma2(pack2(-s, -s), pack2(acc_to_float<kInt8>(a[j]), acc_to_float<kInt8>(a[j + 1])), pack2(r[OFF + j], r[OFF + j + 1]));
+      unpack2(d, r[OFF + j], r[OFF + j + 1]);
     }
   } else {
     float q[4] = {0.f, 0.f, 0.f, 0.f};
@@ -410,7 +394,7 @@ __device__ __forceinline__ void accm_begin(SmemCtl& S, AccRing& ring, uint32_t t
   tmem_ld32u(tbase + ring.slot * kAccCols, a0);
   tmem_wait_ld();
 }
-template <bool kInt8, bool kScore, bool kPacked>
+template <bool kInt8, bool kScore>
 __device__ __forceinline__ void accm_step(SmemCtl& S, AccRing& ring, uint32_t tbase, int lane, uint32_t (&a0)[32],
                                           uint32_t (&a1)[32], float (&r)[64], const float4* gp, const float4 sc,
                                           float (&p)[4], const bool has_next, const bool skip_math) {
@@ -429,7 +413,7 @@ __device__ __forceinline__ void accm_step(SmemCtl& S, AccRing& ring, uint32_t tb
   bool next_ready = true;
   if (has_next) next_ready = mbar_try(smem_u32(&S.acc_full[nslot]), nphase);
   tmem_ld32u(t0 + 32, a1);
-  consume32<kInt8, kScore, kPacked, 0>(a0, r, gp, sc.x, sc.y, p[0], p[1]);
+  consume32<kInt8, kScore, 0>(a0, r, gp, sc.x, sc.y, p[0], p[1]);
   tmem_wait_ld();
   tc_fence_before();
   __syncwarp();
@@ -440,11 +424,11 @@ __device__ __forceinline__ void accm_step(SmemCtl& S, AccRing& ring, uint32_t tb
     tc_fence_after();
     tmem_ld32u(tbase + nslot * kAccCols, a0);
   }
-  consume32<kInt8, kScore, kPacked, 32>(a1, r, gp, sc.z, sc.w, p[2], p[3]);
+  consume32<kInt8, kScore, 32>(a1, r, gp, sc.z, sc.w, p[2], p[3]);
   if (has_next) tmem_wait_ld();
 }
 
-template <bool kInt8, bool kSingle, bool kPacked>
+template <bool kInt8, bool kSingle>
 __global__ void __launch_bounds__(kThreads, 1) sweep_tc_kernel(const __grid_constant__ SweepParams P) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 127) & ~uintptr_t(127));
@@ -693,7 +677,7 @@ __global__ void __launch_bounds__(kThreads, 1) sweep_tc_kernel(const __grid_cons
         accm_begin(S, ring, tbase, a0);
         for (int gi = 0; gi < P.n_fixed_groups; ++gi) {
           const float4 sc = *reinterpret_cast<const float4*>(&S.fixs[gi][hf * 4]);
-          accm_step<kInt8, false, kPacked>(S, ring, tbase, lane, a0, a1, r, gp, sc, p, gi + 1 < P.n_fixed_groups, dbg2);
+          accm_step<kInt8, false>(S, ring, tbase, lane, a0, a1, r, gp, sc, p, gi + 1 < P.n_fixed_groups, dbg2);
         }
       }
       if (P.out != nullptr) {
@@ -722,8 +706,8 @@ __global__ void __launch_bounds__(kThreads, 1) sweep_tc_kernel(const __grid_cons
           const bool noA = (P.cand_noA_mask >> gi) & 1ull;
           const float4 sc = noA ? cb : make_float4(ca.x * cb.x, ca.y * cb.y, ca.z * cb.z, ca.w * cb.w);
           if (ew == 0) TRACE(2, tev, 0);
-          if (gi == P.n_cand_groups - 1) accm_step<kInt8, true, kPacked>(S, ring, tbase, lane, a0, a1, r, gp, sc, p, c + 1 < f.c1, dbg2);
-          else accm_step<kInt8, false, kPacked>(S, ring, tbase, lane, a0, a1, r, gp, sc, p, true, dbg2);
+          if (gi == P.n_cand_groups - 1) accm_step<kInt8, true>(S, ring, tbase, lane, a0, a1, r, gp, sc, p, c + 1 < f.c1, dbg2);
+          else accm_step<kInt8, false>(S, ring, tbase, lane, a0, a1, r, gp, sc, p, true, dbg2);
           if (ew == 0) { TRACE(2, tev, 1); ++tev; }
         }
         const float tot = reduce4_over_rows(p[0], p[1], p[2], p[3], lane);
@@ -789,7 +773,7 @@ __global__ void __launch_bounds__(kThreads, 1) sweep_tc_kernel(const __grid_cons
         acc_begin(S, ring, tbase, a0);
         for (int gi = 0; gi < P.n_fixed_groups; ++gi) {
           const float4 sc = *reinterpret_cast<const float4*>(&S.fixs[gi][hf * 4]);
-          acc_step<kInt8, false, kPacked>(S, ring, tbase, lane, a0, a1, r, g, sc, pdummy, gi + 1 < P.n_fixed_groups, dbg2);
+          acc_step<kInt8, false>(S, ring, tbase, lane, a0, a1, r, g, sc, pdummy, gi + 1 < P.n_fixed_groups, dbg2);
         }
       }
       if (P.out != nullptr) {
@@ -819,7 +803,7 @@ __global__ void __launch_bounds__(kThreads, 1) sweep_tc_kernel(const __grid_cons
           if (ew == 0) TRACE(2, tev, 0);
           const float4 ca = *reinterpret_cast<const float4*>(&S.candA[c][hf * 4]);
           const float4 sc = noA ? cb : make_float4(ca.x * cb.x, ca.y * cb.y, ca.z * cb.z, ca.w * cb.w);
-          acc_step<kInt8, true, kPacked>(S, ring, tbase, lane, a0, a1, r, g, sc, p, c + 1 < f.c1, dbg2);
+          acc_step<kInt8, true>(S, ring, tbase, lane, a0, a1, r, g, sc, p, c + 1 < f.c1, dbg2);
           if (ew == 0) TRACE(2, tev, 1);
           if (P.row_keys) {        // one score per ROW (channel-wise conv search): [tile][candidate][column half][128 rows]
             P.partial[((size_t)f.tile * P.n_cand + c) * 256 + hf * P4V_TILE + quarter * 32 + lane] = (p[0] + p[1]) + (p[2] + p[3]);
@@ -899,22 +883,17 @@ int p4v_launch_sweep_tc(const SweepParams& p_in, const P4VJob* host_jobs, int nu
   if ((kSmemBudget - 2 * (long long)res_bytes - red_bytes - (long long)p.cres_bytes) / per_stage < 3) p.resident_bufs = 1;
   int nst = (int)((kSmemBudget - (long long)p.resident_bufs * res_bytes - red_bytes - (long long)p.cres_bytes) / per_stage);
   if (nst > kMaxStages) nst = kMaxStages;
-  { static const int cap = [] { const char* e = getenv("P4V_MAX_STAGES"); return e ? atoi(e) : 0; }();   // experiment knob
-    if (cap >= 2 && nst > cap) nst = cap; }
   P4V_REQUIRE(nst >= 2, "sweep: operand tiles do not fit the shared-memory ring");
   p.n_stages = nst;
   const size_t smem = (size_t)nst * per_stage + (size_t)p.resident_bufs * res_bytes + p.cres_bytes + ((sizeof(SmemCtl) + 127) & ~size_t(127)) + (size_t)red_bytes + 256;
-#define P4V_LAUNCH(I8, SG, PK)                                                                         \
+#define P4V_LAUNCH(I8, SG)                                                                             \
   do {                                                                                                 \
-    P4V_CUDA_OK(cudaFuncSetAttribute(sweep_tc_kernel<I8, SG, PK>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-    sweep_tc_kernel<I8, SG, PK><<<grid, kThreads, smem, st>>>(p);                                      \
+    P4V_CUDA_OK(cudaFuncSetAttribute(sweep_tc_kernel<I8, SG>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
+    sweep_tc_kernel<I8, SG><<<grid, kThreads, smem, st>>>(p);                                          \
   } while (0)
-#define P4V_LAUNCH2(I8, SG) do { if (packed) P4V_LAUNCH(I8, SG, true); else P4V_LAUNCH(I8, SG, false); } while (0)
   p.debug_mode = g_sweep_debug;
-  static const bool packed = [] { const char* e = getenv("P4V_PACKED"); return e ? atoi(e) != 0 : true; }();
-  if (p.is_int8) { if (single) P4V_LAUNCH2(true, true); else P4V_LAUNCH2(true, false); }
-  else           { if (single) P4V_LAUNCH2(false, true); else P4V_LAUNCH2(false, false); }
-#undef P4V_LAUNCH2
+  if (p.is_int8) { if (single) P4V_LAUNCH(true, true); else P4V_LAUNCH(true, false); }
+  else           { if (single) P4V_LAUNCH(false, true); else P4V_LAUNCH(false, false); }
 #undef P4V_LAUNCH
   P4V_CUDA_OK(cudaGetLastError());
   return 0;
